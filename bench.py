@@ -26,6 +26,10 @@ One "step" = one pass of the hot path over that batch: one transient launch per 
 
 Launch: `python bench.py --gpus N --steps K --warmup W`; for N > 1 under torchrun (one rank per GPU, instances
 sharded by rank, no collective on the data path; totals all-reduced at the end).
+
+`--dump-outputs DIR` (e.g. bench_out/) writes what the last timed step returned for a fixed sample of instances, so that two
+builds can be compared output for output (dump_outputs).  bench.py writes nothing into the tree it runs from: kernels it
+compiles or tunes at run time go to a temporary directory (private_kernel_cache).
 """
 from __future__ import annotations
 
@@ -36,15 +40,19 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 DECKS = ("rc", "rlc")
+DUMP_SAMPLE = 1 << 16       # instances per deck in --dump-outputs: at most (4 x 7 + 3) x 8 bytes each, under 33 MB for rc + rlc
+DUMP_SEED = 2024
 
 
 def load_workloads():
@@ -209,6 +217,33 @@ def host_threads() -> int:
         return os.cpu_count() or 1
 
 
+def private_kernel_cache() -> tempfile.TemporaryDirectory:
+    """A temporary kernel-cache directory holding a link to every file of the pre-built cache (build() ->
+    toy-spice_b200/_kcache, or $TSB_KCACHE).  The library reads the pre-built cubins through the links and puts what it
+    compiles or tunes at run time (NVRTC cubins, launch-bounds choices) there, each file renamed into place over any link
+    of that name, so the tree bench.py runs from is only read and may be read-only.  Removed when the process exits."""
+    src = os.path.abspath(os.environ.get("TSB_KCACHE") or os.path.join(ROOT, "toy-spice_b200", "_kcache"))
+    tmp = tempfile.TemporaryDirectory(prefix="tsb_kcache_")
+    if os.path.isdir(src):
+        for f in os.listdir(src):
+            os.symlink(os.path.join(src, f), os.path.join(tmp.name, f))
+    return tmp
+
+
+def dump_outputs(out_dir: str, decks, n: int) -> None:
+    """--dump-outputs: what the last run of every deck's batch returned to its caller -- statistics [4: min, max, sum, last]
+    [result column][instance], stored rows and status per instance -- for a fixed sample of instances (DUMP_SAMPLE drawn
+    with DUMP_SEED, ascending), as float64 arrays in out_dir/<deck>_{stats,rows,status}.npy; <deck>_instance.npy holds the
+    sampled instance indices."""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, min(n, DUMP_SAMPLE), replace=False))
+    for d in decks:
+        b = d["b_res"]
+        arrays = {"stats": b.stats_all()[:, :, idx], "rows": b.rows()[idx], "status": b.status()[idx], "instance": idx}
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, f"{d['name']}_{name}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 # --------------------------------------------------------------------------------------------
 def cpu_sample(O, W, target_seconds: float, threads: int):
     """Time the CPU oracle on a bounded sample of the SAME workload (same decks, same draws).  Device table from the
@@ -295,7 +330,10 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the per-BASELINE-config entries and the strong-scaling entry")
     ap.add_argument("--config-scale", type=float, default=1.0, help="scale the instance counts of the `configs` / `strong` entries")
     ap.add_argument("--strict-fp", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step (sampled instances) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the results of the GPU path: not with --impl reference")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -314,6 +352,8 @@ def main():
     W = importlib.import_module("toy-spice_b200.workloads")
     S = importlib.import_module("toy-spice_b200.sharding")
     ctx = T.Context(local)
+    kcache = private_kernel_cache()
+    ctx.set_cache_dir(kcache.name)
     stream = torch.cuda.Stream(device=local)
     ctx.set_stream(stream.cuda_stream)
     opts = T.default_opts(strict_fp=args.strict_fp)
@@ -424,6 +464,8 @@ def main():
     t_local = sum(ms_steps) * 1e-3
     t_job, (acc_job, solves_job, exec_job) = S.reduce_job(t_local, [acc_local, solves_local, exec_local], device=dev_name)
     value = acc_job * args.steps / t_job if t_job > 0 else 0.0
+    if args.dump_outputs:
+        dump_outputs(os.path.join(args.dump_outputs, f"rank{rank}") if world > 1 else args.dump_outputs, decks, n)
 
     # ---- timed: end to end through the public API with host buffers -----------------------------
     step_e2e(0); step_e2e(1)

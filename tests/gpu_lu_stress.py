@@ -1,7 +1,6 @@
 """Development driver (not a pytest file): 750 strict-build runs of the warp-per-circuit LU (n = 1..8, 257 systems) against
 the oracle with the device allocator dirtied by NaN-filled buffers in between — hunts for reads of uninitialised memory."""
-import sys, numpy as np, torch
-sys.path.insert(0,'/root/repo/tests'); sys.path.insert(0,'/root/repo')
+import numpy as np, torch
 import parity_util as PU
 from test_lu_operator import mna_like
 T,O=PU.T,PU.O

@@ -5,6 +5,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -48,12 +49,90 @@ def test_recorded_reference_arm_line():
     check_line(json.load(open(os.path.join(ROOT, "profiles", "bench_r01_final_reference_arm.json"))), reference=True)
 
 
+def load_bench():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    B = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(B)
+    return B
+
+
+def check_dump(out_dir, n):
+    """--dump-outputs: float64 arrays only, 64 MB at most, the sampled instances' statistics / rows / status of rc and rlc."""
+    files = sorted(os.listdir(out_dir))
+    assert files == sorted(f"{deck}_{a}.npy" for deck in ("rc", "rlc") for a in ("stats", "rows", "status", "instance")), files
+    assert sum(os.path.getsize(os.path.join(out_dir, f)) for f in files) <= 64 << 20
+    arr = {f[:-4]: np.load(os.path.join(out_dir, f)) for f in files}
+    assert all(a.dtype == np.float64 for a in arr.values())
+    k = min(n, 1 << 16)
+    for deck, ncol in (("rc", 5), ("rlc", 7)):
+        idx = arr[f"{deck}_instance"]
+        assert idx.shape == (k,) and np.all(np.diff(idx) > 0) and idx[0] >= 0 and idx[-1] < n
+        assert arr[f"{deck}_stats"].shape == (4, ncol, k) and arr[f"{deck}_rows"].shape == (k,) and arr[f"{deck}_status"].shape == (k,)
+    return arr
+
+
+def test_dump_outputs_with_stand_in_batches(tmp_path):
+    """dump_outputs on the CPU: batches whose results are known functions of the instance index, so the sample can be checked
+    value for value; the same call twice gives the same files."""
+    B = load_bench()
+
+    class StandIn:
+        def __init__(self, n, ncol):
+            self.n, self.ncol = n, ncol
+
+        def stats_all(self):
+            return np.arange(4 * self.ncol * self.n, dtype=np.float64).reshape(4, self.ncol, self.n)
+
+        def rows(self):
+            return np.arange(self.n, dtype=np.int64) + 300
+
+        def status(self):
+            return (np.arange(self.n) % 3 == 0).astype(np.int32)
+
+    n = 100_000
+    decks = [dict(name="rc", b_res=StandIn(n, 5)), dict(name="rlc", b_res=StandIn(n, 7))]
+    B.dump_outputs(str(tmp_path / "a"), decks, n)
+    B.dump_outputs(str(tmp_path / "b"), decks, n)
+    arr = check_dump(tmp_path / "a", n)
+    for name, a in arr.items():
+        assert np.array_equal(a, np.load(tmp_path / "b" / f"{name}.npy")), name
+    for d in decks:
+        idx = arr[d["name"] + "_instance"].astype(np.int64)
+        assert np.array_equal(arr[d["name"] + "_stats"], d["b_res"].stats_all()[:, :, idx])
+        assert np.array_equal(arr[d["name"] + "_rows"], idx + 300) and np.array_equal(arr[d["name"] + "_status"], idx % 3 == 0)
+
+
+def test_private_kernel_cache_leaves_the_prebuilt_cache_untouched(tmp_path, monkeypatch):
+    """The kernel cache bench.py hands the library: every pre-built file readable through it, and a file the library writes
+    (under a private name, then renamed into place) replaces the link, not the pre-built file."""
+    B = load_bench()
+    src = tmp_path / "kcache"
+    src.mkdir()
+    (src / "k.cubin").write_bytes(b"prebuilt")
+    (src / "k.auto").write_text("3\n")
+    monkeypatch.setenv("TSB_KCACHE", str(src))
+    cache = B.private_kernel_cache()
+    d = cache.name
+    assert not d.startswith(ROOT) and sorted(os.listdir(d)) == ["k.auto", "k.cubin"]
+    assert open(os.path.join(d, "k.cubin"), "rb").read() == b"prebuilt"
+    with open(os.path.join(d, "k.auto.tmp1"), "w") as f:
+        f.write("5\n")
+    os.rename(os.path.join(d, "k.auto.tmp1"), os.path.join(d, "k.auto"))
+    assert (src / "k.auto").read_text() == "3\n" and open(os.path.join(d, "k.auto")).read() == "5\n"
+    cache.cleanup()
+    assert not os.path.exists(d) and sorted(os.listdir(src)) == ["k.auto", "k.cubin"]
+
+
 @pytest.mark.gpu
-def test_live_bench_line(built):
+def test_live_bench_line(built, tmp_path):
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "3", "--instances", "65536", "--no-cpu-baseline",
-                        "--config-scale", "0.004"],
+                        "--config-scale", "0.004", "--dump-outputs", str(tmp_path / "out")],
                        capture_output=True, text=True, timeout=900)
     assert r.returncode == 0, r.stderr[-2000:]
+    arr = check_dump(tmp_path / "out", 65536)
+    for deck in ("rc", "rlc"):
+        assert np.all(arr[f"{deck}_status"] == 0) and np.all(arr[f"{deck}_rows"] > 0) and np.isfinite(arr[f"{deck}_stats"]).all()
     d = json.loads(r.stdout.strip().splitlines()[-1])
     d["cpu_baseline"] = d["cpu_baseline"] or {"value": 1.0, "unit": "", "cores": 1, "kind": "port", "sample": "skipped"}
     check_line(d)
@@ -80,13 +159,10 @@ def test_operator_lu_entry_with_a_stand_in_context(built):
     nominal matrix (tsb_lu_order, host only), the call shape of tsb_lu_solve_batched_dev, the figures it derives — with a
     stand-in context that solves the systems with torch.linalg.solve where the real one launches csrc/lu_warp.cu."""
     import gc
-    import importlib.util
     import time
 
     import torch
-    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
-    B = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(B)
+    B = load_bench()
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     import parity_util as PU
 
