@@ -346,7 +346,13 @@ int tsb_job_result_summary(tsb_job* job, double* out, int64_t* rows_total, int64
  * pivot-row broadcast by warp shuffles (csrc/lu_warp.cu).  Layout: instance-major, A[inst][row][col] row-major
  * (0-based), b[inst][row], x[inst][col]; status[inst] = 0, or 1 for a zero pivot ("matrix factorization failed").
  * pivot_row[k] / pivot_col[k] (k = 0..n-1): 1-based external row / column eliminated at step k+1.
- * strict_fp = 1 reproduces Sparse 1.3's rounding (no FMA contraction, IEEE reciprocals, spSolve's summation order). */
+ * strict_fp = 1 reproduces Sparse 1.3's rounding (no FMA contraction, IEEE reciprocals, spSolve's summation order; a -0.0
+ * entry of A counts as +0.0, as AddElement onto a cleared element makes it).
+ * x of a status-1 system is unspecified (the reference leaves no solution).  Non-finite data is data: an infinite pivot has
+ * the reciprocal 0 in both builds (x of its column = 0).  The fast build's reciprocals come from a flush-to-zero seed:
+ * subnormal pivots and pivots above 2^1022 in magnitude lose accuracy there (the strict build divides).
+ * Refusals, before anything is launched or written: n outside 1..32 (TSB_E_INVALID; tsb_lu_solve_batched_dev:
+ * TSB_E_UNSUPPORTED), a pivot order that is not a permutation of 1..n (TSB_E_INVALID).  n_inst = 0 is a no-op (TSB_OK). */
 /* The reference's symbolic pass on a nominal matrix: the order its first Factor() picks (Markowitz products over the
  * structurally dense matrix, relative threshold 1e-3, diagonal preference; SURVEY Appendix C), Translate numbering =
  * row-major first touch.  Host only (ctx not needed). */
