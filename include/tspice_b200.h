@@ -369,6 +369,25 @@ int tsb_lu_solve_batched(tsb_ctx* ctx, int n, const int* pivot_row, const int* p
 /* Same with every array already in HBM (device pointers); asynchronous on the context's stream. */
 int tsb_lu_solve_batched_dev(tsb_ctx* ctx, int n, const int* pivot_row, const int* pivot_col, uint64_t A_dev, uint64_t b_dev,
                              uint64_t x_dev, uint64_t status_dev, int64_t n_inst, int strict_fp);
+/* Complex systems: the reference's FactorComplex + SolveComplex (pkg/matrix/circuit.go:130, 140), i.e. one AC frequency
+ * point of a host that stamps itself, over a batch.  Layout: interleaved complex, A[inst][row][col][re, im],
+ * b[inst][row][re, im], x[inst][col][re, im] — the layout of C99 double _Complex, std::complex<double>, Go's complex128 and
+ * torch.complex128 (x is the solution vector itself, not the analysis read-out of tsb_run_ac).  The pivot order, n, status
+ * and the refusals are those of tsb_lu_solve_batched.  In the reference the AC order is the one its real operating point
+ * froze (ac.go:33-49): take it from tsb_lu_order on the REAL nominal matrix (e.g. the conductance part G), or from
+ * tsb_plan_structure; no order is chosen on complex values.  A pivot is zero when |re| + |im| == 0 (status 1; x of that
+ * system is unspecified).
+ * strict_fp = 1 reproduces Sparse 1.3's complex arithmetic bit for bit: CMPLX_RECIPROCAL as Smith's scaled division with its
+ * branch predicates, CMPLX_MULT / CMPLX_MULT_SUBT_ASSIGN without contraction, forward substitution skipped when both parts
+ * of an entry are zero, back substitution by ascending columns, -0.0 in either part of an entry of A counted as +0.0.
+ * The fast build contracts to FMA, forms multipliers, and takes the two real quotients of Smith's form from the fast
+ * reciprocal (subnormal and huge parts are limited as for the real fast build).  A pivot with one infinite and one finite
+ * part has the reciprocal 0 in both builds (x of its column = 0).  Pointers need 8-byte alignment only. */
+int tsb_lu_solve_batched_complex(tsb_ctx* ctx, int n, const int* pivot_row, const int* pivot_col, const double* A,
+                                 const double* b, double* x, int32_t* status, int64_t n_inst, int strict_fp);
+/* Same with every array already in HBM (device pointers); asynchronous on the context's stream. */
+int tsb_lu_solve_batched_complex_dev(tsb_ctx* ctx, int n, const int* pivot_row, const int* pivot_col, uint64_t A_dev,
+                                     uint64_t b_dev, uint64_t x_dev, uint64_t status_dev, int64_t n_inst, int strict_fp);
 
 /* ---- introspection / build-time support -------------------------------------------------------*/
 /* CUDA source of the kernels specialised for this batch configuration (which parameters vary). */

@@ -17,6 +17,7 @@
 // message text; Go panics (inconsistent DC sweep lengths, dc.go:21-23) become std::invalid_argument.
 // Header-only; link with -ltspice_b200.
 #pragma once
+#include <complex>
 #include <cstdint>
 #include <map>
 #include <memory>
@@ -216,6 +217,22 @@ inline std::vector<double> LuSolveBatched(Context& ctx, int n, const PivotOrder&
     std::vector<double> x((size_t)n_inst * n);
     status.assign((size_t)n_inst, 0);
     if (tsb_lu_solve_batched(ctx.get(), n, o.row.data(), o.col.data(), A.data(), b.data(), x.data(), status.data(), n_inst, strict ? 1 : 0) != TSB_OK)
+        throw Error(ctx.last_error());
+    return x;
+}
+// Complex systems (FactorComplex + SolveComplex): A [n_inst][n][n], b [n_inst][n] as std::complex<double> (interleaved re, im);
+// returns x [n_inst][n].  The order is the real one: LuOrder on the real nominal matrix, or the plan's.
+inline std::vector<std::complex<double>> LuSolveBatchedComplex(Context& ctx, int n, const PivotOrder& o,
+                                                               const std::vector<std::complex<double>>& A,
+                                                               const std::vector<std::complex<double>>& b,
+                                                               std::vector<int32_t>& status, bool strict = false) {
+    const int64_t n_inst = (int64_t)b.size() / n;
+    if ((int64_t)A.size() != n_inst * n * n) throw std::invalid_argument("A must be n_inst*n*n");
+    std::vector<std::complex<double>> x((size_t)n_inst * n);
+    status.assign((size_t)n_inst, 0);
+    if (tsb_lu_solve_batched_complex(ctx.get(), n, o.row.data(), o.col.data(), reinterpret_cast<const double*>(A.data()),
+                                     reinterpret_cast<const double*>(b.data()), reinterpret_cast<double*>(x.data()), status.data(),
+                                     n_inst, strict ? 1 : 0) != TSB_OK)
         throw Error(ctx.last_error());
     return x;
 }

@@ -48,6 +48,7 @@ ABI_SYMBOLS = [
     "tsb_job_shard", "tsb_job_plan", "tsb_job_set_param", "tsb_job_set_param_uniform", "tsb_job_run_op", "tsb_job_run_tran",
     "tsb_job_run_dc", "tsb_job_sync", "tsb_job_result_status", "tsb_job_result_rows", "tsb_job_result_stats",
     "tsb_job_result_waveform", "tsb_job_result_summary", "tsb_run_ac", "tsb_plan_analysis2",
+    "tsb_lu_solve_batched_complex", "tsb_lu_solve_batched_complex_dev",
 ]
 
 
@@ -155,6 +156,8 @@ def lib():
             "tsb_lu_order": (i32, [i32, P(dbl), P(i32), P(i32)]),
             "tsb_lu_solve_batched": (i32, [vp, i32, P(i32), P(i32), P(dbl), P(dbl), P(dbl), P(C.c_int32), i64, i32]),
             "tsb_lu_solve_batched_dev": (i32, [vp, i32, P(i32), P(i32), u64, u64, u64, u64, i64, i32]),
+            "tsb_lu_solve_batched_complex": (i32, [vp, i32, P(i32), P(i32), P(dbl), P(dbl), P(dbl), P(C.c_int32), i64, i32]),
+            "tsb_lu_solve_batched_complex_dev": (i32, [vp, i32, P(i32), P(i32), u64, u64, u64, u64, i64, i32]),
         }
         for name, (res, args) in sig.items():
             fn = getattr(L, name)
@@ -260,6 +263,32 @@ class Context:
         ip = C.POINTER(C.c_int)
         self._check(lib().tsb_lu_solve_batched_dev(self.h, n, pr.ctypes.data_as(ip), pc.ctypes.data_as(ip), A_ptr, b_ptr, x_ptr,
                                                    status_ptr, n_inst, int(strict)), "tsb_lu_solve_batched_dev")
+
+    def lu_solve_batched_complex(self, A: np.ndarray, b: np.ndarray, order, strict: bool = False):
+        """Complex systems (tsb_lu_solve_batched_complex: FactorComplex + SolveComplex): A [n_inst, n, n], b [n_inst, n]
+        complex128 host arrays -> (x [n_inst, n] complex128, status [n_inst]).  `order` as for lu_solve_batched, frozen on
+        the real nominal matrix (lu_order) or taken from Circuit.structure()."""
+        A = np.ascontiguousarray(A, dtype=np.complex128); b = np.ascontiguousarray(b, dtype=np.complex128)
+        n_inst, n = b.shape
+        pr = np.ascontiguousarray(order[0], dtype=np.int32); pc = np.ascontiguousarray(order[1], dtype=np.int32)
+        x = np.zeros((n_inst, n), dtype=np.complex128); st = np.zeros(n_inst, dtype=np.int32)
+        dp, ip = C.POINTER(C.c_double), C.POINTER(C.c_int)
+        self._check(lib().tsb_lu_solve_batched_complex(self.h, n, pr.ctypes.data_as(ip), pc.ctypes.data_as(ip),
+                                                       A.ctypes.data_as(dp), b.ctypes.data_as(dp), x.ctypes.data_as(dp),
+                                                       st.ctypes.data_as(C.POINTER(C.c_int32)), n_inst, int(strict)),
+                    "tsb_lu_solve_batched_complex")
+        return x, st
+
+    def lu_solve_batched_complex_dev(self, n: int, n_inst: int, A_ptr: int, b_ptr: int, x_ptr: int, status_ptr: int, order,
+                                     strict: bool = False):
+        """Same with device pointers to interleaved complex data (e.g. complex128 tensors' data_ptr()); asynchronous on the
+        context's stream, which is first ordered after torch's current stream."""
+        self.wait_torch_stream()
+        pr = np.ascontiguousarray(order[0], dtype=np.int32); pc = np.ascontiguousarray(order[1], dtype=np.int32)
+        ip = C.POINTER(C.c_int)
+        self._check(lib().tsb_lu_solve_batched_complex_dev(self.h, n, pr.ctypes.data_as(ip), pc.ctypes.data_as(ip), A_ptr, b_ptr,
+                                                           x_ptr, status_ptr, n_inst, int(strict)),
+                    "tsb_lu_solve_batched_complex_dev")
 
     def close(self):
         if self.h:

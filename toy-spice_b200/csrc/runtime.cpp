@@ -28,6 +28,8 @@ cudaError_t launch_fill_i64(long long* p, long long n, long long v, int sms, cud
 cudaError_t launch_summary(const double* stats, long long n_inst, int ncol, double* partial, int blocks_x, cudaStream_t s);
 cudaError_t launch_lu_warp(const double* A, const double* b, double* x, int* status, long long n_inst, int n, const int* prow,
                            const int* pcol, int strict, int sms, cudaStream_t s);
+cudaError_t launch_clu_warp(const double* A, const double* b, double* x, int* status, long long n_inst, int n, const int* prow,
+                            const int* pcol, int strict, int sms, cudaStream_t s);
 }
 
 using namespace tsb;
@@ -1551,8 +1553,13 @@ static int lu_check_order(tsb_ctx* ctx, int n, const int* pr, const int* pc, int
     return TSB_OK;
 }
 
-int tsb_lu_solve_batched_dev(tsb_ctx* ctx, int n, const int* pivot_row, const int* pivot_col, uint64_t A_dev, uint64_t b_dev,
-                             uint64_t x_dev, uint64_t status_dev, int64_t n_inst, int strict_fp) {
+// Real (words = 1) and complex (words = 2: interleaved re, im) systems share the checks, the launch accounting and the host
+// staging; only the kernel family differs.
+typedef cudaError_t (*LuLaunch)(const double*, const double*, double*, int*, long long, int, const int*, const int*, int, int,
+                                cudaStream_t);
+
+static int lu_solve_dev(tsb_ctx* ctx, LuLaunch launch, int n, const int* pivot_row, const int* pivot_col, uint64_t A_dev,
+                        uint64_t b_dev, uint64_t x_dev, uint64_t status_dev, int64_t n_inst, int strict_fp) {
     if (!ctx) return TSB_E_CUDA;
     if (!pivot_row || !pivot_col || !A_dev || !b_dev || !x_dev || !status_dev || n_inst < 0) return TSB_E_INVALID;
     int h[64];
@@ -1561,37 +1568,59 @@ int tsb_lu_solve_batched_dev(tsb_ctx* ctx, int n, const int* pivot_row, const in
     if (n_inst == 0) return TSB_OK;
     CU(ctx, cudaSetDevice(ctx->device));
     // the pivot order goes to the kernel by value (a kernel parameter): nothing to allocate or copy per call
-    cudaError_t e = launch_lu_warp((const double*)(uintptr_t)A_dev, (const double*)(uintptr_t)b_dev, (double*)(uintptr_t)x_dev,
-                                   (int*)(uintptr_t)status_dev, n_inst, n, h, h + 32, strict_fp != 0, ctx->sms, ctx->stream);
+    cudaError_t e = launch((const double*)(uintptr_t)A_dev, (const double*)(uintptr_t)b_dev, (double*)(uintptr_t)x_dev,
+                           (int*)(uintptr_t)status_dev, n_inst, n, h, h + 32, strict_fp != 0, ctx->sms, ctx->stream);
     ++ctx->launches;
     CU(ctx, e);
     return TSB_OK;
 }
 
-int tsb_lu_solve_batched(tsb_ctx* ctx, int n, const int* pivot_row, const int* pivot_col, const double* A, const double* b,
-                         double* x, int32_t* status, int64_t n_inst, int strict_fp) {
+static int lu_solve_host(tsb_ctx* ctx, LuLaunch launch, int words, const char* what, int n, const int* pivot_row,
+                         const int* pivot_col, const double* A, const double* b, double* x, int32_t* status, int64_t n_inst,
+                         int strict_fp) {
     if (!ctx) return TSB_E_CUDA;
     if (!A || !b || !x || !status || n_inst < 0 || n < 1 || n > 32) return TSB_E_INVALID;
     if (n_inst == 0) return TSB_OK;
     CU(ctx, cudaSetDevice(ctx->device));
-    const size_t na = (size_t)n_inst * n * n * sizeof(double), nb = (size_t)n_inst * n * sizeof(double);
+    const size_t na = (size_t)n_inst * n * n * words * sizeof(double), nb = (size_t)n_inst * n * words * sizeof(double);
     double *dA = nullptr, *db = nullptr, *dx = nullptr; int* dst = nullptr;
     CU(ctx, cudaMalloc(&dA, na));
     if (cudaMalloc(&db, nb) != cudaSuccess || cudaMalloc(&dx, nb) != cudaSuccess || cudaMalloc(&dst, (size_t)n_inst * sizeof(int)) != cudaSuccess) {
         cudaFree(dA); cudaFree(db); cudaFree(dx); cudaFree(dst); cudaGetLastError();
-        return fail(ctx, TSB_E_NOMEM, "tsb_lu_solve_batched: out of device memory");
+        return fail(ctx, TSB_E_NOMEM, std::string(what) + ": out of device memory");
     }
     int rc = TSB_OK;
     if (cudaMemcpyAsync(dA, A, na, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess ||
         cudaMemcpyAsync(db, b, nb, cudaMemcpyHostToDevice, ctx->stream) != cudaSuccess) rc = fail(ctx, TSB_E_CUDA, "H2D copy failed");
-    if (rc == TSB_OK) rc = tsb_lu_solve_batched_dev(ctx, n, pivot_row, pivot_col, (uint64_t)(uintptr_t)dA, (uint64_t)(uintptr_t)db,
-                                                    (uint64_t)(uintptr_t)dx, (uint64_t)(uintptr_t)dst, n_inst, strict_fp);
+    if (rc == TSB_OK) rc = lu_solve_dev(ctx, launch, n, pivot_row, pivot_col, (uint64_t)(uintptr_t)dA, (uint64_t)(uintptr_t)db,
+                                        (uint64_t)(uintptr_t)dx, (uint64_t)(uintptr_t)dst, n_inst, strict_fp);
     if (rc == TSB_OK && (cudaMemcpyAsync(x, dx, nb, cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess ||
                          cudaMemcpyAsync(status, dst, (size_t)n_inst * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess ||
                          cudaStreamSynchronize(ctx->stream) != cudaSuccess))
-        rc = fail(ctx, TSB_E_CUDA, std::string("tsb_lu_solve_batched: ") + cudaGetErrorString(cudaGetLastError()));
+        rc = fail(ctx, TSB_E_CUDA, std::string(what) + ": " + cudaGetErrorString(cudaGetLastError()));
     cudaFree(dA); cudaFree(db); cudaFree(dx); cudaFree(dst);
     return rc;
+}
+
+int tsb_lu_solve_batched_dev(tsb_ctx* ctx, int n, const int* pivot_row, const int* pivot_col, uint64_t A_dev, uint64_t b_dev,
+                             uint64_t x_dev, uint64_t status_dev, int64_t n_inst, int strict_fp) {
+    return lu_solve_dev(ctx, launch_lu_warp, n, pivot_row, pivot_col, A_dev, b_dev, x_dev, status_dev, n_inst, strict_fp);
+}
+
+int tsb_lu_solve_batched(tsb_ctx* ctx, int n, const int* pivot_row, const int* pivot_col, const double* A, const double* b,
+                         double* x, int32_t* status, int64_t n_inst, int strict_fp) {
+    return lu_solve_host(ctx, launch_lu_warp, 1, "tsb_lu_solve_batched", n, pivot_row, pivot_col, A, b, x, status, n_inst, strict_fp);
+}
+
+int tsb_lu_solve_batched_complex_dev(tsb_ctx* ctx, int n, const int* pivot_row, const int* pivot_col, uint64_t A_dev,
+                                     uint64_t b_dev, uint64_t x_dev, uint64_t status_dev, int64_t n_inst, int strict_fp) {
+    return lu_solve_dev(ctx, launch_clu_warp, n, pivot_row, pivot_col, A_dev, b_dev, x_dev, status_dev, n_inst, strict_fp);
+}
+
+int tsb_lu_solve_batched_complex(tsb_ctx* ctx, int n, const int* pivot_row, const int* pivot_col, const double* A,
+                                 const double* b, double* x, int32_t* status, int64_t n_inst, int strict_fp) {
+    return lu_solve_host(ctx, launch_clu_warp, 2, "tsb_lu_solve_batched_complex", n, pivot_row, pivot_col, A, b, x, status,
+                         n_inst, strict_fp);
 }
 
 // ---- introspection -------------------------------------------------------------------------------
