@@ -32,7 +32,7 @@ type base struct {
 	GPU     int                    // device ordinal
 	N       int64                  // instances (default 1)
 	Sweep   map[ParamRef][]float64 // per-instance parameter values, N each
-	Out     int                    // TSB_OUT_WAVE (default) | TSB_OUT_STATS | TSB_OUT_GRID
+	Out     int                    // TSB_OUT_WAVE (default) | TSB_OUT_STATS | TSB_OUT_GRID | TSB_OUT_MEAS
 
 	ctx   *Context
 	plan  *Plan

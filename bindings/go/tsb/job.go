@@ -17,8 +17,9 @@ import (
 )
 
 type Job struct {
-	h *C.tsb_job
-	N int64
+	h     *C.tsb_job
+	N     int64
+	nMeas int
 }
 
 func NewJob(gpus []int, netlistText string, n int64) (*Job, error) {
@@ -32,7 +33,7 @@ func NewJob(gpus []int, netlistText string, n int64) (*Job, error) {
 	if rc := C.tsb_job_create(&ids[0], C.int(len(ids)), cs, C.int64_t(n), &h); rc != C.TSB_OK {
 		return nil, fmt.Errorf("tsb_job_create: %s", C.GoString(C.tsb_last_error(nil)))
 	}
-	return &Job{h, n}, nil
+	return &Job{h: h, N: n}, nil
 }
 
 func (j *Job) Close() { C.tsb_job_destroy(j.h); j.h = nil }
@@ -81,6 +82,34 @@ func (j *Job) Summary(nColumns int) (min, max, sum []float64, rows int64, totals
 		totals[k] = int64(t[k])
 	}
 	return buf[:nColumns], buf[nColumns : 2*nColumns], buf[2*nColumns:], int64(r), totals, nil
+}
+
+// SetMeasures sets the measurement table of every GPU's shard.
+func (j *Job) SetMeasures(m []Meas) error {
+	t := measTable(m)
+	var p *C.tsb_meas
+	if len(t) > 0 {
+		p = &t[0]
+	}
+	if rc := C.tsb_job_set_measures(j.h, p, C.int(len(t))); rc != C.TSB_OK {
+		return j.err("tsb_job_set_measures")
+	}
+	j.nMeas = len(t)
+	return nil
+}
+
+// Measures returns value[m][instance] and abscissa[m][instance] in job order.
+func (j *Job) Measures() (value, abscissa [][]float64, err error) {
+	flat := make([]float64, 2*int64(j.nMeas)*j.N+1)
+	if rc := C.tsb_job_result_measures(j.h, (*C.double)(unsafe.Pointer(&flat[0]))); rc != C.TSB_OK {
+		return nil, nil, j.err("tsb_job_result_measures")
+	}
+	value, abscissa = make([][]float64, j.nMeas), make([][]float64, j.nMeas)
+	for m := 0; m < j.nMeas; m++ {
+		value[m] = flat[int64(m)*j.N : int64(m+1)*j.N]
+		abscissa[m] = flat[int64(j.nMeas+m)*j.N : int64(j.nMeas+m+1)*j.N]
+	}
+	return value, abscissa, nil
 }
 
 func (j *Job) Status() ([]int32, error) {

@@ -141,9 +141,10 @@ type ParamRef struct {
 
 // Batch is N instances of a plan (tsb_batch).
 type Batch struct {
-	h    *C.tsb_batch
-	plan *Plan
-	N    int64
+	h     *C.tsb_batch
+	plan  *Plan
+	N     int64
+	nMeas int
 }
 
 func NewBatch(plan *Plan, n int64) (*Batch, error) {
@@ -151,7 +152,7 @@ func NewBatch(plan *Plan, n int64) (*Batch, error) {
 	if rc := C.tsb_batch_create(plan.h, C.int64_t(n), &h); rc != C.TSB_OK {
 		return nil, plan.ctx.lastErr("tsb_batch_create")
 	}
-	b := &Batch{h, plan, n}
+	b := &Batch{h: h, plan: plan, N: n}
 	runtime.SetFinalizer(b, func(b *Batch) { b.Close() })
 	return b, nil
 }
@@ -226,6 +227,50 @@ func (b *Batch) Instance(i int64, analysis int) (map[string][]float64, error) {
 		out[name] = s
 	}
 	return out, nil
+}
+
+// Meas is one entry of a measurement table (tsb_meas; the .meas family: WHEN, AT, MAX, MIN, AVG, INTEG, RMS, defined
+// in tspice_b200.h).  From / To = math.Inf(-1) / math.Inf(1): the whole series.
+type Meas struct {
+	Kind, Column, TrigColumn, Edge, Count int
+	Level, From, To                       float64
+}
+
+func measTable(m []Meas) []C.tsb_meas {
+	t := make([]C.tsb_meas, len(m))
+	for k, e := range m {
+		t[k] = C.tsb_meas{kind: C.int(e.Kind), column: C.int(e.Column), trig_column: C.int(e.TrigColumn), edge: C.int(e.Edge),
+			count: C.int(e.Count), level: C.double(e.Level), from: C.double(e.From), to: C.double(e.To)}
+	}
+	return t
+}
+
+// SetMeasures sets the batch's measurement table (copied; nil clears); runs with TSB_OUT_MEAS reduce it on the device.
+func (b *Batch) SetMeasures(m []Meas) error {
+	t := measTable(m)
+	var p *C.tsb_meas
+	if len(t) > 0 {
+		p = &t[0]
+	}
+	if rc := C.tsb_batch_set_measures(b.h, p, C.int(len(t))); rc != C.TSB_OK {
+		return b.plan.ctx.lastErr("tsb_batch_set_measures")
+	}
+	b.nMeas = len(t)
+	return nil
+}
+
+// Measures returns value[m][instance] and abscissa[m][instance] of the last TSB_OUT_MEAS run.
+func (b *Batch) Measures() (value, abscissa [][]float64, err error) {
+	flat := make([]float64, 2*int64(b.nMeas)*b.N+1)
+	if rc := C.tsb_result_measures(b.h, (*C.double)(unsafe.Pointer(&flat[0]))); rc != C.TSB_OK {
+		return nil, nil, b.plan.ctx.lastErr("tsb_result_measures")
+	}
+	value, abscissa = make([][]float64, b.nMeas), make([][]float64, b.nMeas)
+	for m := 0; m < b.nMeas; m++ {
+		value[m] = flat[int64(m)*b.N : int64(m+1)*b.N]
+		abscissa[m] = flat[int64(b.nMeas+m)*b.N : int64(b.nMeas+m+1)*b.N]
+	}
+	return value, abscissa, nil
 }
 
 // Stats returns min / max / sum / last per column and instance: stats[q][column][instance] (TSB_OUT_STATS runs).

@@ -156,8 +156,49 @@ enum {
                            (solution[i], solution[i+Size]) (matrix/circuit.go:168-173) while the vector is laid out
                            solution[2k] = re x_k, solution[2k+1] = im x_k (:41-44, :85-97).  Default (flag clear): entry i is
                            (re x_i, im x_i) — what the accessor means if the module returns split halves.  The module's
-                           source is not available, so both read-outs are offered (DESIGN.md, quirk Q28). */
+                           source is not available, so both read-outs are offered (DESIGN.md, quirk Q28). */,
+    TSB_OUT_MEAS = 16   /* tsb_run_tran / tsb_run_dc / tsb_run_ac: the measurements of the batch's measurement table
+                           (tsb_batch_set_measures), reduced on the device from the stored rows as they are produced;
+                           read with tsb_result_measures.  Implies TSB_OUT_STATS; combines with WAVE and GRID. */
 };
+
+/* ---- measurements (the SPICE .meas family, reduced on the device) -------------------------------------------------
+ * The series of one instance is its stored rows (x_r, y_r), r = 0 .. last: exactly the rows TSB_OUT_WAVE would write,
+ * rows beyond wave_cap_rows included; x is column 0 (TIME / SWEEP1 / FREQ), y is `column`.  Every operation below is
+ * individually rounded in both builds, so a result is a function of the stored rows alone (independent of strict_fp,
+ * the mapping, the processing order, lane refill and the shared time grid).
+ *   WHEN   segment (r, r+1) rises when t_r < L <= t_r+1 and falls when t_r > L >= t_r+1 (t = trig_column, L = level; a
+ *          NaN sample never crosses); CROSS is either.  f = (L - t_r) / (t_r+1 - t_r), x* = x_r + f (x_r+1 - x_r),
+ *          value = y_r + f (y_r+1 - y_r).  Crossings with from <= x* <= to count; the result is (value, x*) of the
+ *          count-th (1-based) or, count = -1, of the last one; (NaN, NaN) when there is none.  A delay (TRIG / TARG) is
+ *          the difference of two WHEN abscissas.
+ *   AT     r+1 = the first row with x_r+1 >= level: value = y_r+1 if x_r+1 == level, else
+ *          y_r + ((level - x_r) / (x_r+1 - x_r)) (y_r+1 - y_r).  Result (value, level); value NaN for a level outside
+ *          [x_0, x_last].
+ *   MAX / MIN   over the rows with from <= x_r <= to, NaN samples ignored, a tie goes to the first row: (extreme, its x_r);
+ *          (NaN, NaN) when no row is in the window.
+ *   INTEG / AVG / RMS   window [a, b]: a = x_0 if from = -inf else from, b = x_last if to = +inf else to; NaN when
+ *          a < x_0, b > x_last (an instance that failed before the window ended) or a > b.  Trapezoid rule over the
+ *          segments clipped to [a, b] (an endpoint inside a segment takes its value as AT does), summed in row order
+ *          from 0.0: INTEG = sum (x_hi - x_lo) (y_lo + y_hi) 0.5, AVG = INTEG / (b - a),
+ *          RMS = sqrt(sum (x_hi - x_lo) (y_lo^2 + y_hi^2) 0.5 / (b - a)).  Abscissa NaN.  Zero width: INTEG 0, AVG and
+ *          RMS NaN.
+ * Kind, column and trig_column are compiled into the kernels (a new set of them compiles once, NVRTC); level, count,
+ * edge and the window are run-time arguments.  Refused (before anything is launched): TSB_OUT_MEAS without a table or with
+ * a column outside 1 .. n_columns-1 of the analysis (TSB_E_INVALID), on the nested DC sweep or with an explicit
+ * coop_parts > 0 (TSB_E_UNSUPPORTED); coop_parts = -1 takes the thread-per-circuit mapping. */
+enum { TSB_MEAS_WHEN = 0, TSB_MEAS_AT = 1, TSB_MEAS_MAX = 2, TSB_MEAS_MIN = 3, TSB_MEAS_AVG = 4, TSB_MEAS_INTEG = 5, TSB_MEAS_RMS = 6 };
+enum { TSB_EDGE_CROSS = 0, TSB_EDGE_RISE = 1, TSB_EDGE_FALL = 2 };
+enum { TSB_MEAS_CAP = 16 };
+typedef struct tsb_meas {
+    int kind;
+    int column;        /* result column measured, 1 .. n_columns-1 of the analysis (tsb_plan_column_name) */
+    int trig_column;   /* WHEN: the column whose crossing is sought (may equal `column`) */
+    int edge;          /* WHEN: TSB_EDGE_* */
+    int count;         /* WHEN: the count-th such crossing, 1-based; -1 = the last one */
+    double level;      /* WHEN: crossing level; AT: the abscissa */
+    double from, to;   /* window on column 0; -inf / +inf = the whole series */
+} tsb_meas;
 
 void tsb_default_opts(tsb_opts* o);
 const char* tsb_version(void);
@@ -245,6 +286,12 @@ int tsb_batch_set_param_uniform(tsb_batch* batch, int dev, int param, double val
  * do not change by a bit.  NULL removes the order. */
 int tsb_batch_set_order(tsb_batch* batch, const int64_t* perm);
 
+/* Measurement table of the batch (copied; n_meas <= TSB_MEAS_CAP; (NULL, 0) clears).  TSB_E_INVALID for an unknown kind, a
+ * column or trig_column < 1, a NaN window or from > to, and for WHEN / AT a NaN level, for WHEN an unknown edge or count 0.
+ * The columns are checked against the analysis when a run selects TSB_OUT_MEAS.  Setting a table discards the measurements
+ * of the last run (tsb_result_measures fails until the next TSB_OUT_MEAS run). */
+int tsb_batch_set_measures(tsb_batch* batch, const tsb_meas* m, int n_meas);
+
 /* Analyses — the batch equivalents of analysis.NewOP / NewTransient / NewDCSweep + Setup + Execute. */
 int tsb_run_op(tsb_batch* batch, const tsb_opts* opts);
 int tsb_run_tran(tsb_batch* batch, double tstart, double tstop, double tstep, double tmax, int uic,
@@ -299,6 +346,9 @@ int tsb_result_waveform(tsb_batch* batch, int64_t inst, double* out, int64_t cap
 /* Whole wave / stats arrays in the device layout above. */
 int tsb_result_wave_all(tsb_batch* batch, double* out, int64_t n_doubles);
 int tsb_result_stats_all(tsb_batch* batch, double* out /*[4][n_columns][n_inst]*/);
+/* Measurements of the last run (TSB_OUT_MEAS): out[0][m][inst] = value, out[1][m][inst] = abscissa, for the table the run
+ * used.  TSB_E_INVALID after a run without measurements. */
+int tsb_result_measures(tsb_batch* batch, double* out /*[2][n_meas][n_inst]*/);
 /* Batch totals computed on the GPU: sum over instances of accepted steps, rejected steps, transient solves,
  * OP solves (reference-equivalent counts) and executed factor+solve passes. */
 int tsb_result_totals(tsb_batch* batch, int64_t totals[5]);
@@ -335,6 +385,8 @@ int tsb_job_sync(tsb_job* job);
 int tsb_job_result_status(tsb_job* job, int32_t* status /*[n_inst]*/);
 int tsb_job_result_rows(tsb_job* job, int64_t* rows /*[n_inst]*/);
 int tsb_job_result_stats(tsb_job* job, double* stats /*[4][n_columns][n_inst]*/);
+int tsb_job_set_measures(tsb_job* job, const tsb_meas* m, int n_meas);
+int tsb_job_result_measures(tsb_job* job, double* out /*[2][n_meas][n_inst], JOB order*/);
 int tsb_job_result_waveform(tsb_job* job, int64_t inst, double* out, int64_t cap_rows, int64_t* n_rows);
 /* out[3][n_columns] (min, max, sum), stored rows and the five totals of tsb_result_totals, merged over the GPUs. */
 int tsb_job_result_summary(tsb_job* job, double* out, int64_t* rows_total, int64_t totals[5]);
@@ -394,7 +446,8 @@ int tsb_lu_solve_batched_complex_dev(tsb_ctx* ctx, int n, const int* pivot_row, 
 int tsb_batch_kernel_source(tsb_batch* batch, const tsb_opts* opts, char* buf, int64_t cap, int64_t* needed);
 /* Which specialisation the two calls below describe: dc_src_dev >= 0 selects the DC-sweep kernel for that source
  * (dc_src2_dev >= 0: the nested sweep), grid != 0 the TSB_OUT_GRID kernels; (-1, -1, 0) = the default OP / transient
- * kernels.  A batch used this way is for introspection only (build step), do not run analyses on it. */
+ * kernels.  The bit TSB_OUT_MEAS in `grid` selects the kernels of the batch's measurement table instead (grid ==
+ * TSB_OUT_MEAS) or in addition (grid == TSB_OUT_GRID | TSB_OUT_MEAS).  A batch used this way is for introspection only (build step), do not run analyses on it. */
 int tsb_batch_kernel_variant(tsb_batch* batch, int dc_src_dev, int dc_src2_dev, int grid);
 /* Cache key (hex) of that source + compile options; the cubin is looked up as <cache_dir>/<key>.cubin. */
 int tsb_batch_kernel_key(tsb_batch* batch, const tsb_opts* opts, char* buf, int cap);

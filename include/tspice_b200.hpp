@@ -83,12 +83,24 @@ public:
         if ((int64_t)values.size() != n_) throw std::invalid_argument("values must have one entry per instance");
         if (tsb_batch_set_param(h_, d, param, values.data()) != TSB_OK) throw Error(ckt_->ctx().last_error());
     }
+    // Measurement table (TSB_OUT_MEAS; definitions in tspice_b200.h); an empty vector clears it.
+    void SetMeasures(const std::vector<tsb_meas>& m) {
+        if (tsb_batch_set_measures(h_, m.empty() ? nullptr : m.data(), (int)m.size()) != TSB_OK) throw Error(ckt_->ctx().last_error());
+        n_meas_ = (int)m.size();
+    }
+    // [2: value, abscissa][n_meas][n_inst] of the last run with TSB_OUT_MEAS.
+    std::vector<double> Measures() const {
+        std::vector<double> out((size_t)2 * n_meas_ * n_);
+        if (tsb_result_measures(h_, out.data()) != TSB_OK) throw Error(ckt_->ctx().last_error());
+        return out;
+    }
     tsb_batch* get() const { return h_; }
     Circuit& circuit() const { return *ckt_; }
     int64_t size() const { return n_; }
 private:
     Circuit* ckt_;
     int64_t n_;
+    int n_meas_ = 0;
     tsb_batch* h_ = nullptr;
 };
 
@@ -152,7 +164,7 @@ class Transient : public Analysis {
 public:
     Transient(double tStart, double tStop, double tStep, double tMax, bool uic)
         : tStart_(tStart), tStop_(tStop), tStep_(tStep), tMax_(tMax), uic_(uic) {}
-    int out = TSB_OUT_WAVE;      // TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_GRID (results resampled onto a fixed time grid)
+    int out = TSB_OUT_WAVE;      // TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_GRID (results resampled onto a fixed time grid) | TSB_OUT_MEAS
     int64_t cap_rows = 16384;
     double grid_dt = 0.0;        // TSB_OUT_GRID: grid spacing (0: the clamped tStep)
     void Execute() override {

@@ -26,7 +26,9 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
 
 AN_OP, AN_TRAN, AN_AC, AN_DC, AN_DC2 = 0, 1, 2, 3, 4
-OUT_WAVE, OUT_STATS, OUT_GRID, OUT_AC_REFREAD = 1, 2, 4, 8
+OUT_WAVE, OUT_STATS, OUT_GRID, OUT_AC_REFREAD, OUT_MEAS = 1, 2, 4, 8, 16
+MEAS_WHEN, MEAS_AT, MEAS_MAX, MEAS_MIN, MEAS_AVG, MEAS_INTEG, MEAS_RMS = range(7)
+EDGE_CROSS, EDGE_RISE, EDGE_FALL = range(3)
 K_R, K_C, K_L, K_V, K_I, K_D, K_Q, K_M, K_K, K_LCORE = range(10)
 ST_OK, ST_OP_FAILED, ST_TRAN_FAILED, ST_DC_FAILED, ST_OVERFLOW, ST_AC_FAILED = range(6)
 
@@ -48,7 +50,8 @@ ABI_SYMBOLS = [
     "tsb_job_shard", "tsb_job_plan", "tsb_job_set_param", "tsb_job_set_param_uniform", "tsb_job_run_op", "tsb_job_run_tran",
     "tsb_job_run_dc", "tsb_job_sync", "tsb_job_result_status", "tsb_job_result_rows", "tsb_job_result_stats",
     "tsb_job_result_waveform", "tsb_job_result_summary", "tsb_run_ac", "tsb_plan_analysis2",
-    "tsb_lu_solve_batched_complex", "tsb_lu_solve_batched_complex_dev",
+    "tsb_lu_solve_batched_complex", "tsb_lu_solve_batched_complex_dev", "tsb_batch_set_measures", "tsb_result_measures",
+    "tsb_job_set_measures", "tsb_job_result_measures",
 ]
 
 
@@ -60,6 +63,23 @@ class Opts(C.Structure):
     _fields_ = [("max_iter", C.c_int), ("abstol", C.c_double), ("reltol", C.c_double), ("gmin", C.c_double),
                 ("trtol", C.c_double), ("strict_fp", C.c_int), ("block_size", C.c_int), ("skip_linear_resolve", C.c_int), ("min_blocks", C.c_int), ("lane_refill", C.c_int), ("grid_dt", C.c_double),
                 ("share_time_grid", C.c_int), ("coop_parts", C.c_int)]
+
+
+class Meas(C.Structure):
+    """One entry of a measurement table (tsb_meas; definitions in include/tspice_b200.h).  `from_` is the window's start."""
+    _fields_ = [("kind", C.c_int), ("column", C.c_int), ("trig_column", C.c_int), ("edge", C.c_int), ("count", C.c_int),
+                ("level", C.c_double), ("from_", C.c_double), ("to", C.c_double)]
+
+
+def meas(kind: int, column: int, level: float = 0.0, trig_column: int | None = None, edge: int = EDGE_CROSS, count: int = 1,
+         from_: float = -np.inf, to: float = np.inf) -> Meas:
+    """A measurement-table entry; trig_column defaults to `column`."""
+    return Meas(kind, column, column if trig_column is None else trig_column, edge, count, level, from_, to)
+
+
+def _meas_table(measures):
+    arr = (Meas * max(1, len(measures)))(*measures)
+    return (arr if measures else None), len(measures)
 
 
 def lib_path() -> str:
@@ -126,6 +146,10 @@ def lib():
             "tsb_result_waveform": (i32, [vp, i64, P(dbl), i64, P(i64)]),
             "tsb_result_wave_all": (i32, [vp, P(dbl), i64]),
             "tsb_result_stats_all": (i32, [vp, P(dbl)]),
+            "tsb_batch_set_measures": (i32, [vp, P(Meas), i32]),
+            "tsb_result_measures": (i32, [vp, P(dbl)]),
+            "tsb_job_set_measures": (i32, [vp, P(Meas), i32]),
+            "tsb_job_result_measures": (i32, [vp, P(dbl)]),
             "tsb_result_totals": (i32, [vp, P(i64)]),
             "tsb_batch_kernel_source": (i32, [vp, P(Opts), C.c_char_p, i64, P(i64)]),
             "tsb_batch_kernel_key": (i32, [vp, P(Opts), C.c_char_p, i32]),
@@ -496,11 +520,13 @@ class Batch:
             self._check(lib().tsb_batch_set_param(self.h, d, param, v.ctypes.data_as(C.POINTER(C.c_double))), "set_param")
 
     # -- kernel introspection -------------------------------------------------------------------
-    def kernel_variant(self, dc_src=-1, dc_src2=-1, grid=False):
-        """Select the specialisation kernel_source / kernel_key describe (introspection-only batches; build step)."""
+    def kernel_variant(self, dc_src=-1, dc_src2=-1, grid=False, meas=False):
+        """Select the specialisation kernel_source / kernel_key describe (introspection-only batches; build step);
+        meas=True: the kernels of the batch's measurement table."""
         d1 = self._dev(dc_src) if dc_src != -1 else -1
         d2 = self._dev(dc_src2) if dc_src2 != -1 else -1
-        self._check(lib().tsb_batch_kernel_variant(self.h, d1, d2, int(bool(grid))), "tsb_batch_kernel_variant")
+        flags = (1 if grid else 0) | (OUT_MEAS if meas else 0)
+        self._check(lib().tsb_batch_kernel_variant(self.h, d1, d2, flags), "tsb_batch_kernel_variant")
 
     def kernel_source(self, opts: Opts | None = None) -> str:
         need = C.c_int64()
@@ -536,6 +562,13 @@ class Batch:
         """AC analysis of a linear circuit (tsb_run_ac): sweep 'DEC' | 'OCT' | 'LIN', n_points frequencies in total."""
         st = {"DEC": 0, "OCT": 1, "LIN": 2}[sweep.upper()]
         self._check(lib().tsb_run_ac(self.h, st, int(n_points), fstart, fstop, out, C.byref(opts) if opts is not None else None), "tsb_run_ac")
+
+    def set_measures(self, measures):
+        """Measurement table (tsb_batch_set_measures): a list of Meas (see meas()); [] clears.  Runs with OUT_MEAS use it."""
+        self.n_meas = 0
+        tab, n = _meas_table(list(measures))
+        self._check(lib().tsb_batch_set_measures(self.h, tab, n), "tsb_batch_set_measures")
+        self.n_meas = n
 
     def set_order(self, perm):
         """Processing order (tsb_batch_set_order): slot s works on instance perm[s]; None removes it."""
@@ -600,6 +633,12 @@ class Batch:
         n, ncol, _ = self.dims()
         out = np.zeros((4, ncol, n)) if out is None else out
         self._check(lib().tsb_result_stats_all(self.h, out.ctypes.data_as(C.POINTER(C.c_double))), "result_stats_all")
+        return out
+
+    def measures(self) -> np.ndarray:
+        """[2: value, abscissa][n_meas][n_inst] of the last run (OUT_MEAS)."""
+        out = np.zeros((2, getattr(self, "n_meas", 0), self.n_inst))
+        self._check(lib().tsb_result_measures(self.h, out.ctypes.data_as(C.POINTER(C.c_double))), "result_measures")
         return out
 
     def fetch_async(self, stats=None, rows=None, status=None, counters=None):
@@ -668,6 +707,19 @@ class Job:
         if v.shape != (self.n_inst,):
             raise ValueError("values must have shape [n_inst]")
         self._check(lib().tsb_job_set_param(self.h, d, param, v.ctypes.data_as(C.POINTER(C.c_double))), "job_set_param")
+
+    def set_measures(self, measures):
+        """Measurement table of every shard (tsb_job_set_measures)."""
+        self.n_meas = 0
+        tab, n = _meas_table(list(measures))
+        self._check(lib().tsb_job_set_measures(self.h, tab, n), "job_set_measures")
+        self.n_meas = n
+
+    def measures(self) -> np.ndarray:
+        """[2: value, abscissa][n_meas][n_inst] in job order."""
+        out = np.zeros((2, getattr(self, "n_meas", 0), self.n_inst))
+        self._check(lib().tsb_job_result_measures(self.h, out.ctypes.data_as(C.POINTER(C.c_double))), "job_result_measures")
+        return out
 
     def run_op(self, opts: Opts | None = None):
         self._check(lib().tsb_job_run_op(self.h, C.byref(opts) if opts is not None else None), "job_run_op")

@@ -968,6 +968,13 @@ std::string generate_source(const Plan& pl, const CodegenConfig& cfg) {
     const CoopPlan* coop = nullptr;          // cooperative transient kernels ride along (device/coop.cuh)
     if (cfg.coop_parts > 0 && cfg.fast_div) { auto it = pl.coop.find(cfg.coop_parts); if (it != pl.coop.end()) coop = &it->second; }
     if (coop) e.line("#define TSB_COOP 1");
+    if (!cfg.meas.empty()) {             // measurement table: the compile-time half (skeleton.cuh, TsbSink::emit_meas)
+        std::string spec;
+        for (size_t k = 0; k + 2 < cfg.meas.size(); k += 3)
+            spec += (k ? ", {" : "{") + std::to_string(cfg.meas[k]) + ", " + std::to_string(cfg.meas[k + 1]) + ", " + std::to_string(cfg.meas[k + 2]) + "}";
+        e.line("#define TSB_MEAS " + std::to_string(cfg.meas.size() / 3));
+        e.line("#define TSB_MEAS_SPEC " + spec);
+    }
     if (!cfg.extra_defines.empty()) e.os << cfg.extra_defines << "\n";     // development knob ($TSB_EXTRA_DEFINES)
     e.os << k_models_src << "\n" << k_skeleton_src << "\n";
 

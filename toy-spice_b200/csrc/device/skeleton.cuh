@@ -69,6 +69,12 @@ struct TsbArgs {
     // tsb_optran, which then hands the device state and the solution over — [n_state + N + 1][n_inst] doubles — instead of
     // running the transient itself; tsb_coop_tran picks them up.  NULL: tsb_optran runs the whole analysis.
     double* coop_state;
+    // TSB_OUT_MEAS (kernels generated with TSB_MEAS): the run-time half of the measurement table — kind, column and trigger
+    // column are compile-time (tsb_meas_spec), so a new level or window reuses the kernel.  Appended: every field above
+    // keeps its offset.
+    double meas_level[16], meas_from[16], meas_to[16];
+    int meas_count[16], meas_edge[16];
+    double* meas_out;          // [2][n_meas][n_inst]: value, abscissa
 };
 
 // Slot -> instance.  With an order, lanes of a warp can be given instances that behave alike (similar Newton
@@ -89,6 +95,7 @@ __device__ __forceinline__ long long tsb_slot_instance(const TsbArgs& a, long lo
 #define TSB_OUT_STATS 2
 #define TSB_OUT_GRID 4
 #define TSB_OUT_AC_REFREAD 8
+#define TSB_OUT_MEAS 16
 
 #ifndef TSB_COOP
 #define TSB_COOP 0
@@ -156,6 +163,35 @@ __device__ __forceinline__ bool tsb_converged_dc(const double* x, const double* 
     return ok;
 }
 
+// Measurements (TSB_OUT_MEAS, the SPICE .meas family; definitions in include/tspice_b200.h).  Kernels generated for a
+// measurement table define TSB_MEAS (its length) and TSB_MEAS_SPEC ({kind, column, trigger column} per entry): the sink
+// walks the table at compile time, so every column index into the row — a register array — is a literal.  Every
+// operation is individually rounded in both builds, so a result depends on the stored rows only.
+#ifndef TSB_MEAS
+#define TSB_MEAS 0
+#endif
+#define TSB_MEAS_WHEN 0
+#define TSB_MEAS_AT 1
+#define TSB_MEAS_MAX 2
+#define TSB_MEAS_MIN 3
+#define TSB_MEAS_AVG 4
+#define TSB_MEAS_INTEG 5
+#define TSB_MEAS_RMS 6
+#define TSB_EDGE_RISE 1
+#define TSB_EDGE_FALL 2
+#if TSB_MEAS
+struct TsbMeasSpec { int kind, col, tcol; };
+__host__ __device__ constexpr TsbMeasSpec tsb_meas_spec(int i) {
+    constexpr TsbMeasSpec t[TSB_MEAS] = {TSB_MEAS_SPEC};
+    return t[i];
+}
+// The value at abscissa L of the segment (x0, y0) - (x1, y1) with x0 < L <= x1, as AT defines it.
+__device__ __forceinline__ double tsb_meas_interp(double x0, double y0, double x1, double y1, double L) {
+    if (L == x1) return y1;
+    return __dadd_rn(y0, __dmul_rn(__ddiv_rn(__dsub_rn(L, x0), __dsub_rn(x1, x0)), __dsub_rn(y1, y0)));
+}
+#endif
+
 // Result sink of one instance: waveform rows to HBM (instance-fastest layout, so a warp whose
 // lanes are at the same row index writes 256 contiguous bytes per column) and running
 // min / max / sum / last per column in shared memory.
@@ -184,7 +220,115 @@ struct TsbSink {
                 sm[(2 * j + 1) * TSB_BLOCK] = make_double2(0.0, 0.0);
             }
         }
+#if TSB_MEAS
+        if (a.out_flags & TSB_OUT_MEAS) meas_begin();
+#endif
     }
+#if TSB_MEAS
+    // Measurement m keeps two double2 per thread after the statistics pairs (same thread-interleaved layout):
+    //   WHEN            {value, abscissa} of the crossing taken, {crossings counted, -}
+    //   AT              {value, -}, {1 once the row at or past the level was seen, -}
+    //   MAX / MIN       {extreme, its abscissa} (NaN: no row in the window yet)
+    //   AVG/INTEG/RMS   {trapezoid sum of y (of y^2 for RMS) over the window, -}
+    // Each step walks the table by template recursion (entry m, then m + 1): m is a literal in every instance.  Entries
+    // whose columns this kernel's rows do not have belong to another analysis (the run checks the table against its own
+    // columns) and compile to nothing here.
+    __device__ __forceinline__ double2* meas_slot(int m) const { return sm + (2 * NCOL + 2 * m) * TSB_BLOCK; }
+    template <int m = 0> __device__ __forceinline__ void meas_begin() {
+        if constexpr (m < TSB_MEAS) {
+            constexpr TsbMeasSpec s = tsb_meas_spec(m);
+            if constexpr (s.col < NCOL && s.tcol < NCOL) {
+                const double nan = __longlong_as_double(0x7ff8000000000000LL);
+                double2* st = meas_slot(m);
+                st[0] = s.kind >= TSB_MEAS_AVG ? make_double2(0.0, 0.0) : make_double2(nan, nan);
+                st[TSB_BLOCK] = make_double2(0.0, 0.0);
+            }
+            meas_begin<m + 1>();
+        }
+    }
+    // One stored row; runs before the statistics update, so the previous row (n_rows > 0) is still in the `last` slots.
+    __device__ __forceinline__ void emit_meas(const double* row) { emit_meas_entry<0>(row, n_rows > 0, sm[1 * TSB_BLOCK].y, row[0]); }
+    template <int m> __device__ __forceinline__ void emit_meas_entry(const double* row, bool prev, double x0, double x1) {
+        if constexpr (m < TSB_MEAS) {
+            constexpr TsbMeasSpec s = tsb_meas_spec(m);
+            if constexpr (s.col < NCOL && s.tcol < NCOL) {
+                double2* st = meas_slot(m);
+                const double y1 = row[s.col];
+                if constexpr (s.kind == TSB_MEAS_WHEN) {
+                    if (prev) {
+                        const double L = a.meas_level[m], t0 = sm[(2 * s.tcol + 1) * TSB_BLOCK].y, t1 = row[s.tcol];
+                        const int edge = a.meas_edge[m];
+                        const bool rise = (t0 < L) & (L <= t1), fall = (t0 > L) & (L >= t1);      // NaN: neither
+                        if ((rise & (edge != TSB_EDGE_FALL)) | (fall & (edge != TSB_EDGE_RISE))) {
+                            const double f = __ddiv_rn(__dsub_rn(L, t0), __dsub_rn(t1, t0));
+                            const double xs = __dadd_rn(x0, __dmul_rn(f, __dsub_rn(x1, x0)));
+                            const int count = a.meas_count[m];
+                            const double seen = st[TSB_BLOCK].x;
+                            if (xs >= a.meas_from[m] && xs <= a.meas_to[m] && (count < 0 || seen < (double)count)) {
+                                st[TSB_BLOCK].x = seen + 1.0;
+                                if (count < 0 || seen + 1.0 == (double)count) {
+                                    const double y0 = sm[(2 * s.col + 1) * TSB_BLOCK].y;
+                                    st[0] = make_double2(__dadd_rn(y0, __dmul_rn(f, __dsub_rn(y1, y0))), xs);
+                                }
+                            }
+                        }
+                    }
+                } else if constexpr (s.kind == TSB_MEAS_AT) {
+                    const double L = a.meas_level[m];
+                    if (st[TSB_BLOCK].x == 0.0 && x1 >= L) {
+                        st[TSB_BLOCK].x = 1.0;
+                        if (prev) st[0].x = tsb_meas_interp(x0, sm[(2 * s.col + 1) * TSB_BLOCK].y, x1, y1, L);
+                        else if (x1 == L) st[0].x = y1;                  // (x_0 > level: outside the series, stays NaN)
+                    }
+                } else if constexpr (s.kind == TSB_MEAS_MAX || s.kind == TSB_MEAS_MIN) {
+                    if (x1 >= a.meas_from[m] && x1 <= a.meas_to[m]) {
+                        const double e = st[0].x;
+                        const bool better = s.kind == TSB_MEAS_MAX ? y1 > e : y1 < e;      // strict: a tie keeps the first row
+                        if (better | ((e != e) & (y1 == y1))) st[0] = make_double2(y1, x1);
+                    }
+                } else {
+                    if (prev) {
+                        const double from = a.meas_from[m], to = a.meas_to[m];
+                        const double lo = x0 > from ? x0 : from, hi = x1 < to ? x1 : to;      // the segment clipped to the window
+                        if (lo < hi) {
+                            const double y0 = sm[(2 * s.col + 1) * TSB_BLOCK].y;
+                            const double ylo = lo == x0 ? y0 : tsb_meas_interp(x0, y0, x1, y1, lo);
+                            const double yhi = tsb_meas_interp(x0, y0, x1, y1, hi);
+                            const double w = __dsub_rn(hi, lo);
+                            const double h = s.kind == TSB_MEAS_RMS ? __dadd_rn(__dmul_rn(ylo, ylo), __dmul_rn(yhi, yhi)) : __dadd_rn(ylo, yhi);
+                            st[0].x = __dadd_rn(st[0].x, __dmul_rn(__dmul_rn(w, h), 0.5));
+                        }
+                    }
+                }
+            }
+            emit_meas_entry<m + 1>(row, prev, x0, x1);
+        }
+    }
+    // xf, xl: column 0 of the first and of the last stored row
+    __device__ __forceinline__ void meas_finish() { meas_finish_entry<0>(sm[0].x, sm[1 * TSB_BLOCK].y); }
+    template <int m> __device__ __forceinline__ void meas_finish_entry(double xf, double xl) {
+        if constexpr (m < TSB_MEAS) {
+            constexpr TsbMeasSpec s = tsb_meas_spec(m);
+            const double nan = __longlong_as_double(0x7ff8000000000000LL);
+            if constexpr (s.col < NCOL && s.tcol < NCOL) {
+                const double2 st = meas_slot(m)[0];
+                double v = st.x, xa = st.y;
+                if constexpr (s.kind == TSB_MEAS_AT) xa = a.meas_level[m];
+                if constexpr (s.kind >= TSB_MEAS_AVG) {
+                    const double from = a.meas_from[m], to = a.meas_to[m];
+                    const double lo = from == -TSB_INF ? xf : from, hi = to == TSB_INF ? xl : to;
+                    xa = nan;
+                    if (n_rows == 0 || lo < xf || hi > xl || lo > hi) v = nan;
+                    else if (s.kind == TSB_MEAS_AVG) v = __ddiv_rn(v, __dsub_rn(hi, lo));
+                    else if (s.kind == TSB_MEAS_RMS) v = __dsqrt_rn(__ddiv_rn(v, __dsub_rn(hi, lo)));
+                }
+                a.meas_out[(long long)m * a.n_inst + inst] = v;
+                a.meas_out[(long long)(TSB_MEAS + m) * a.n_inst + inst] = xa;
+            }
+            meas_finish_entry<m + 1>(xf, xl);
+        }
+    }
+#endif
     __device__ __forceinline__ double grid_time(int k) const {
         const double t = __dadd_rn(a.tstart, __dmul_rn((double)(k + 1), a.grid_dt));   // two roundings in every build (no FMA)
         return t < a.tstop ? t : a.tstop;
@@ -217,6 +361,9 @@ struct TsbSink {
                 for (int j = 0; j < NCOL; ++j) __stcs(w + j * a.n_inst, row[j]);     // streaming store: written once, never re-read
             } else overflow = true;
         }
+#if TSB_MEAS
+        if (a.out_flags & TSB_OUT_MEAS) emit_meas(row);      // TSB_OUT_MEAS implies TSB_OUT_STATS: reads the `last` slots first
+#endif
         if (a.out_flags & TSB_OUT_STATS) {
             if (n_rows == 0) sm[0] = make_double2(row[0], row[0]);     // column 0: the first row, kept in the {min, max} slot
             // running min / max that ignore NaN samples (the accumulators start at +-inf and can never become NaN
@@ -268,6 +415,9 @@ struct TsbSink {
                 ++grid_k;
             }
         }
+#if TSB_MEAS
+        if (a.out_flags & TSB_OUT_MEAS) meas_finish();
+#endif
         if (a.out_flags & TSB_OUT_STATS) {
 #pragma unroll
             for (int j = 0; j < NCOL; ++j) {

@@ -22,6 +22,7 @@ struct tsb_job {
     };
     std::vector<Shard> shards;
     int64_t n_inst = 0;
+    int n_meas = 0;                   // measurement table of every shard (tsb_job_set_measures)
     std::string err;
 };
 
@@ -137,6 +138,30 @@ int tsb_job_result_stats(tsb_job* j, double* stats) {
         rc = tsb_result_stats_all(s.batch, tmp.data());
         if (rc != TSB_OK) return rc;
         for (int k = 0; k < 4 * ncol; ++k) std::memcpy(stats + (size_t)k * j->n_inst + s.lo, tmp.data() + (size_t)k * n, (size_t)n * sizeof(double));
+        return (int)TSB_OK;
+    });
+}
+int tsb_job_set_measures(tsb_job* j, const tsb_meas* m, int n_meas) {
+    if (!j) return TSB_E_INVALID;
+    for (auto& s : j->shards) {
+        int rc = tsb_batch_set_measures(s.batch, m, n_meas);
+        if (rc != TSB_OK) return job_fail(j, rc, tsb_last_error(s.ctx));
+    }
+    j->n_meas = n_meas;
+    return TSB_OK;
+}
+// measurements [2][n_meas][n_inst] in job order (each shard's block is copied row by row into place)
+int tsb_job_result_measures(tsb_job* j, double* out) {
+    if (!j || !out) return TSB_E_INVALID;
+    return for_all_shards(j, [&](tsb_job::Shard& s) {
+        int64_t n = 0;
+        int rc = tsb_result_dims(s.batch, &n, nullptr, nullptr);
+        if (rc != TSB_OK) return rc;
+        const size_t rows = 2 * (size_t)j->n_meas;
+        std::vector<double> tmp(rows * n);
+        rc = tsb_result_measures(s.batch, tmp.data());
+        if (rc != TSB_OK) return rc;
+        for (size_t k = 0; k < rows; ++k) std::memcpy(out + k * j->n_inst + s.lo, tmp.data() + k * n, (size_t)n * sizeof(double));
         return (int)TSB_OK;
     });
 }

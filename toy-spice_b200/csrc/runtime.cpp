@@ -69,6 +69,9 @@ struct TsbArgsHost {
     int tgrid_role;
     double Uc[32];
     double* coop_state;
+    double meas_level[16], meas_from[16], meas_to[16];
+    int meas_count[16], meas_edge[16];
+    double* meas_out;
 };
 
 struct KernelModule {
@@ -153,6 +156,11 @@ struct tsb_batch {
     long long* d_order = nullptr;                      // tsb_batch_set_order: processing order (device copy)
     double* d_coop_state = nullptr;                    // cooperative mapping: hand-over of the operating point, [n_state + n + 1][n_inst]
     size_t wave_bytes = 0, stats_bytes = 0;
+    std::vector<tsb_meas> meas;                        // tsb_batch_set_measures
+    bool meas_kernel = false;                          // the next module request wants the kernels of this table (TSB_MEAS)
+    double* d_meas = nullptr;                          // [2][n_meas][n_inst] of the last TSB_OUT_MEAS run
+    size_t meas_bytes = 0;
+    int meas_last = 0;                                 // measurements the last run produced (0: it had no TSB_OUT_MEAS)
 };
 
 namespace {
@@ -281,6 +289,8 @@ CodegenConfig make_config(const tsb_batch* b, const tsb_opts& o, int dc_param) {
     if (cfg.coop_parts) cfg.tgrid = false;
     if (const char* tf = getenv("TSB_TRANFAST")) cfg.tranfast = *tf != '0';       // development knob: A/B of the condensed elimination
     cfg.grid = b->grid_kernel;
+    if (b->meas_kernel)
+        for (const tsb_meas& m : b->meas) { cfg.meas.push_back(m.kind); cfg.meas.push_back(m.column); cfg.meas.push_back(m.trig_column); }
     cfg.dc_nested = b->dc_nested; cfg.dc_param2 = b->dc_param2;
     cfg.order = b->d_order != nullptr;
     if (const char* x = getenv("TSB_EXTRA_DEFINES")) {          // development knob for A/B kernel experiments
@@ -358,6 +368,8 @@ int get_module(tsb_batch* b, tsb_opts o, int dc_param, KernelModule** out, std::
     snprintf(tail, sizeof tail, "|%d|%d|%d|%d|%d|%d|%d|%d|%d|%d|%d|%d|%lld|%p|", o.coop_parts, o.share_time_grid != 0, o.strict_fp, o.block_size, o.skip_linear_resolve, o.min_blocks, o.lane_refill,
              (int)b->grid_kernel, (int)(b->d_order != nullptr), dc_param, (int)b->dc_nested, b->dc_param2, ctx->choice_epoch, (void*)ctx);
     sig += tail;
+    if (b->meas_kernel)
+        for (const tsb_meas& m : b->meas) sig += std::to_string(m.kind) + "," + std::to_string(m.column) + "," + std::to_string(m.trig_column) + ";";
     if (xd) sig += xd;
     if (const char* tf = getenv("TSB_TRANFAST")) { sig += "|tf"; sig += tf; }
     if (b->memo_module && sig == b->memo_sig) {
@@ -464,7 +476,7 @@ int guard_check(tsb_batch* b) {
     auto name_of = [&](void* p) -> const char* {
         const std::pair<const void*, const char*> known[] = {
             {b->d_wave, "wave"}, {b->d_stats, "stats"}, {b->d_rows, "rows"}, {b->d_status, "status"},
-            {b->d_counters, "counters"}, {b->d_scratch, "scratch"}, {b->d_sweep, "sweep"}};
+            {b->d_counters, "counters"}, {b->d_scratch, "scratch"}, {b->d_sweep, "sweep"}, {b->d_meas, "meas"}};
         for (const auto& kn : known)
             if (p == kn.first) return kn.second;
         return "buffer";
@@ -484,11 +496,12 @@ int guard_check(tsb_batch* b) {
 
 void free_results(tsb_batch* b) {
     gfree(b, b->d_wave); gfree(b, b->d_stats); gfree(b, b->d_rows); gfree(b, b->d_status);
-    gfree(b, b->d_counters); gfree(b, b->d_scratch); gfree(b, b->d_sweep); gfree(b, b->d_sweep2); cudaFree(b->d_totals); cudaFree(b->d_work);
+    gfree(b, b->d_counters); gfree(b, b->d_scratch); gfree(b, b->d_sweep); gfree(b, b->d_sweep2); gfree(b, b->d_meas); cudaFree(b->d_totals); cudaFree(b->d_work);
     b->d_work = nullptr;
     b->d_wave = b->d_stats = b->d_scratch = b->d_sweep = b->d_sweep2 = nullptr;
     b->d_rows = b->d_counters = nullptr; b->d_status = nullptr; b->d_totals = nullptr;
-    b->wave_bytes = b->stats_bytes = 0;
+    b->wave_bytes = b->stats_bytes = b->meas_bytes = 0;
+    b->meas_last = 0;
 }
 
 int alloc_results(tsb_batch* b, int analysis, int out_flags, int64_t cap_rows, int n_sweep) {
@@ -505,6 +518,15 @@ int alloc_results(tsb_batch* b, int analysis, int out_flags, int64_t cap_rows, i
     if (stats_bytes != b->stats_bytes) {
         gfree(b, b->d_stats); b->stats_bytes = 0;
         if (stats_bytes) { CU(ctx, galloc(b, (void**)&b->d_stats, stats_bytes)); b->stats_bytes = stats_bytes; }
+    }
+    b->meas_last = 0;
+    if (out_flags & TSB_OUT_MEAS) {
+        const size_t meas_bytes = (size_t)2 * b->meas.size() * N * sizeof(double);
+        if (meas_bytes != b->meas_bytes) {
+            gfree(b, b->d_meas); b->meas_bytes = 0;
+            CU(ctx, galloc(b, (void**)&b->d_meas, meas_bytes)); b->meas_bytes = meas_bytes;
+        }
+        b->meas_last = (int)b->meas.size();
     }
     if (!b->d_rows) CU(ctx, galloc(b, (void**)&b->d_rows, N * sizeof(long long)));
     if (!b->d_status) CU(ctx, galloc(b, (void**)&b->d_status, N * sizeof(int)));
@@ -534,6 +556,7 @@ int launch(tsb_batch* b, const tsb_opts& o, cudaKernel_t kernel, TsbArgsHost& ar
     int block = o.block_size > 0 ? o.block_size : 128;
     const int ncol_smem = b->plan->p.num_columns(b->analysis == TSB_AN_DC2 ? TSB_AN_DC2 : b->analysis == TSB_AN_AC ? TSB_AN_AC : TSB_AN_TRAN);
     size_t smem = (args.out_flags & (TSB_OUT_STATS | TSB_OUT_GRID)) ? (size_t)4 * ncol_smem * block * sizeof(double) : 0;
+    if (args.out_flags & TSB_OUT_MEAS) smem += (size_t)4 * b->meas_last * block * sizeof(double);     // 32 bytes per measurement
     if (smem > 48 * 1024) CU(ctx, cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     long long blocks = (args.n_run + block - 1) / block;
     if (blocks > 0x7fffffffLL) blocks = 0x7fffffffLL;
@@ -587,6 +610,13 @@ int fill_common(tsb_batch* b, const tsb_opts& o, TsbArgsHost& a) {
     a.counters = b->d_counters; a.scratch = b->d_scratch;
     a.out_flags = b->out_flags; a.cap_rows = b->cap_rows;
     a.skip_linear_resolve = o.skip_linear_resolve;
+    if (b->out_flags & TSB_OUT_MEAS) {
+        for (int m = 0; m < b->meas_last; ++m) {
+            const tsb_meas& t = b->meas[m];
+            a.meas_level[m] = t.level; a.meas_from[m] = t.from; a.meas_to[m] = t.to; a.meas_count[m] = t.count; a.meas_edge[m] = t.edge;
+        }
+        a.meas_out = b->d_meas;
+    }
     return TSB_OK;
 }
 
@@ -612,9 +642,22 @@ tsb_opts resolve(const tsb_opts* o, const Plan& plan) {
 // Per-thread statistics live in shared memory (32 bytes per result column): a circuit with many result columns does not fit
 // 128 threads' worth into an SM's 227 KB.  The block shrinks (whole warps) until it does; the block size is part of the
 // kernel's specialisation, so this happens before the module is requested.
-void fit_block_to_shared_memory(tsb_opts& o, int ncol, int out_flags) {
+void fit_block_to_shared_memory(tsb_opts& o, int ncol, int out_flags, int n_meas) {
     if (!(out_flags & (TSB_OUT_STATS | TSB_OUT_GRID))) return;
-    while (o.block_size > 32 && (size_t)4 * ncol * o.block_size * sizeof(double) > (size_t)226 * 1024) o.block_size -= 32;
+    const int slots = ncol + ((out_flags & TSB_OUT_MEAS) ? n_meas : 0);      // a measurement takes 32 bytes, as a column does
+    while (o.block_size > 32 && (size_t)4 * slots * o.block_size * sizeof(double) > (size_t)226 * 1024) o.block_size -= 32;
+}
+
+// TSB_OUT_MEAS: the table is checked against the columns of the analysis before anything is allocated or launched.
+int check_measures(tsb_batch* b, int analysis, int out_flags) {
+    if (!(out_flags & TSB_OUT_MEAS)) return TSB_OK;
+    if (b->meas.empty()) return fail(b->ctx, TSB_E_INVALID, "TSB_OUT_MEAS: the batch has no measurement table (tsb_batch_set_measures)");
+    const int ncol = b->plan->p.num_columns(analysis);
+    for (const tsb_meas& m : b->meas)
+        if (m.column >= ncol || m.trig_column >= ncol)
+            return fail(b->ctx, TSB_E_INVALID, "TSB_OUT_MEAS: measurement column " + std::to_string(m.column >= ncol ? m.column : m.trig_column) +
+                                                   " is out of range for the analysis (" + std::to_string(ncol) + " columns)");
+    return TSB_OK;
 }
 
 // Launch-bounds autotuning.  The spill rule above is a static prior; what it trades (resident warps against spilled
@@ -1116,9 +1159,11 @@ int tsb_run_tran(tsb_batch* b, double tstart, double tstop, double tstep, double
     int rc = check_batch(b); if (rc != TSB_OK) return rc;
     tsb_ctx* ctx = b->ctx;
     if (!(tstop > 0) || !(tstep > 0)) return fail(ctx, TSB_E_INVALID, "tstop and tstep must be positive");
-    if (!(out_flags & (TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_GRID))) return fail(ctx, TSB_E_INVALID, "no output selected");
+    if (!(out_flags & (TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_GRID | TSB_OUT_MEAS))) return fail(ctx, TSB_E_INVALID, "no output selected");
     if ((out_flags & TSB_OUT_WAVE) && (out_flags & TSB_OUT_GRID)) return fail(ctx, TSB_E_INVALID, "TSB_OUT_WAVE and TSB_OUT_GRID share the waveform buffer: select one");
     if ((out_flags & TSB_OUT_WAVE) && wave_cap_rows <= 0) return fail(ctx, TSB_E_INVALID, "wave_cap_rows must be positive");
+    if ((rc = check_measures(b, TSB_AN_TRAN, out_flags)) != TSB_OK) return rc;
+    if (out_flags & TSB_OUT_MEAS) out_flags |= TSB_OUT_STATS;     // the previous stored row lives in the statistics' `last` slots
     tsb_opts o = resolve(opts, b->plan->p);
     // NewTransient (tran.go:29-55)
     if (tstep > tstop / 300) tstep = tstop / 300;
@@ -1144,7 +1189,7 @@ int tsb_run_tran(tsb_batch* b, double tstart, double tstop, double tstep, double
         // needs holds; otherwise thread-per-circuit
         const Plan& cpl = b->plan->p;
         o.coop_parts = 0;
-        if (!cpl.has_bjt && !cpl.has_mutual && !o.strict_fp && !(out_flags & TSB_OUT_GRID) && o.skip_linear_resolve && !o.lane_refill) {
+        if (!cpl.has_bjt && !cpl.has_mutual && !o.strict_fp && !(out_flags & (TSB_OUT_GRID | TSB_OUT_MEAS)) && o.skip_linear_resolve && !o.lane_refill) {
             // two parts where they fit; more parts only when the statistics of fewer do not leave an SM two blocks
             if (cpl.n() >= TSB_COOP_AUTO_MIN_N)
                 for (int pick : {2, 4, 8}) {
@@ -1162,14 +1207,16 @@ int tsb_run_tran(tsb_batch* b, double tstart, double tstop, double tstep, double
         if (!cpl.coop.count(o.coop_parts)) return fail(ctx, TSB_E_UNSUPPORTED, "coop_parts: the netlist has no partition into that many sub-circuits (tsb_plan_coop_info)");
         if (o.strict_fp) return fail(ctx, TSB_E_UNSUPPORTED, "coop_parts: the nested-dissection order is a re-association, not available in the strict build");
         if (out_flags & TSB_OUT_GRID) return fail(ctx, TSB_E_UNSUPPORTED, "coop_parts: TSB_OUT_GRID is not available on the cooperative mapping");
+        if (out_flags & TSB_OUT_MEAS) return fail(ctx, TSB_E_UNSUPPORTED, "coop_parts: TSB_OUT_MEAS is not available on the cooperative mapping");
         if (!o.skip_linear_resolve || o.lane_refill) return fail(ctx, TSB_E_UNSUPPORTED, "coop_parts needs skip_linear_resolve = 1 and lane_refill = 0");
         if (o.min_blocks <= 0) o.min_blocks = 2;          // tsb_optran only runs the operating point here: no launch-bounds search
-    } else fit_block_to_shared_memory(o, b->plan->p.num_columns(TSB_AN_TRAN), out_flags);
+    } else fit_block_to_shared_memory(o, b->plan->p.num_columns(TSB_AN_TRAN), out_flags, (int)b->meas.size());
     KernelModule* m = nullptr;
     b->grid_kernel = (out_flags & TSB_OUT_GRID) != 0;
+    b->meas_kernel = (out_flags & TSB_OUT_MEAS) != 0;
     std::string autokey;
     rc = get_module(b, o, -1, &m, &autokey);
-    if (rc != TSB_OK) { b->grid_kernel = false; return rc; }
+    if (rc != TSB_OK) { b->grid_kernel = b->meas_kernel = false; return rc; }
     if ((rc = alloc_results(b, TSB_AN_TRAN, out_flags, (out_flags & (TSB_OUT_WAVE | TSB_OUT_GRID)) ? wave_cap_rows : 0, 0)) != TSB_OK) return rc;
     TsbArgsHost a;
     if ((rc = fill_common(b, o, a)) != TSB_OK) return rc;
@@ -1184,9 +1231,9 @@ int tsb_run_tran(tsb_batch* b, double tstart, double tstop, double tstep, double
         !(tune_env && *tune_env == '0') && cap == cudaStreamCaptureStatusNone) {
         rc = autotune_min_blocks(b, o, autokey, m->min_blocks, a, persistent);
         if (rc == TSB_OK) rc = get_module(b, o, -1, &m);
-        if (rc != TSB_OK) { b->grid_kernel = false; return rc; }
+        if (rc != TSB_OK) { b->grid_kernel = b->meas_kernel = false; return rc; }
     }
-    b->grid_kernel = false;
+    b->grid_kernel = b->meas_kernel = false;
     b->tgrid_used = 0;
     const Plan& pl = b->plan->p;
     if (o.coop_parts > 0) {
@@ -1239,7 +1286,10 @@ static int run_dc_impl(tsb_batch* b, int src_dev, double start, double stop, dou
         return fail(ctx, TSB_E_INVALID, nested ? "source not found" : "source not found");       // dc.go:47-68, :226-228
     if (!(inc > 0) || (nested && !(inc2 > 0))) return fail(ctx, TSB_E_INVALID, "sweep increment must be positive");
     if (out_flags & TSB_OUT_GRID) return fail(ctx, TSB_E_INVALID, "TSB_OUT_GRID applies to transient analysis only");
-    if (!(out_flags & (TSB_OUT_WAVE | TSB_OUT_STATS))) return fail(ctx, TSB_E_INVALID, "no output selected");
+    if (!(out_flags & (TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_MEAS))) return fail(ctx, TSB_E_INVALID, "no output selected");
+    if (nested && (out_flags & TSB_OUT_MEAS)) return fail(ctx, TSB_E_UNSUPPORTED, "TSB_OUT_MEAS: the nested DC sweep's column 0 is not monotone");
+    if ((rc = check_measures(b, TSB_AN_DC, out_flags)) != TSB_OK) return rc;
+    if (out_flags & TSB_OUT_MEAS) out_flags |= TSB_OUT_STATS;
     std::vector<double> s1, s2;
     for (double v = start; v <= stop; v += inc) { s1.push_back(v); if (s1.size() > (1u << 24)) break; }   // dc.go:36-42
     if (nested) for (double v = start2; v <= stop2; v += inc2) { s2.push_back(v); if (s2.size() > (1u << 24)) break; }
@@ -1251,7 +1301,7 @@ static int run_dc_impl(tsb_batch* b, int src_dev, double start, double stop, dou
     }
     tsb_opts o = resolve(opts, b->plan->p);
     o.coop_parts = 0;          // the cooperative mapping is a transient-only specialisation
-    fit_block_to_shared_memory(o, p.num_columns(nested ? (int)TSB_AN_DC2 : (int)TSB_AN_DC), out_flags);
+    fit_block_to_shared_memory(o, p.num_columns(nested ? (int)TSB_AN_DC2 : (int)TSB_AN_DC), out_flags, (int)b->meas.size());
     CU(ctx, cudaSetDevice(ctx->device));
     auto dc_param_of = [&](int d) {
         const Dev& sd = p.devs[d];
@@ -1263,9 +1313,9 @@ static int run_dc_impl(tsb_batch* b, int src_dev, double start, double stop, dou
         return fail(ctx, TSB_E_INVALID, "the swept source value is set per instance");
     const int an = nested ? (int)TSB_AN_DC2 : (int)TSB_AN_DC;
     KernelModule* m = nullptr;
-    b->dc_nested = nested; b->dc_param2 = dc_param2;
+    b->dc_nested = nested; b->dc_param2 = dc_param2; b->meas_kernel = (out_flags & TSB_OUT_MEAS) != 0;
     rc = get_module(b, o, dc_param, &m);
-    b->dc_nested = false; b->dc_param2 = -1;
+    b->dc_nested = false; b->dc_param2 = -1; b->meas_kernel = false;
     if (rc != TSB_OK) return rc;
     if ((rc = alloc_results(b, an, out_flags, (out_flags & TSB_OUT_WAVE) ? (int64_t)sweep.size() : 0, (int)sweep.size())) != TSB_OK) return rc;
     TsbArgsHost a;
@@ -1299,15 +1349,20 @@ int tsb_run_ac(tsb_batch* b, int sweep_type, int n_points, double fstart, double
                                              ":126-150); that state is an artefact of the un-vendored sparse module and is not reproduced");
     if (sweep_type < 0 || sweep_type > 2 || n_points < 1 || n_points > (1 << 20)) return fail(ctx, TSB_E_INVALID, "invalid sweep type or number of points");
     if (out_flags & TSB_OUT_GRID) return fail(ctx, TSB_E_INVALID, "TSB_OUT_GRID applies to transient analysis only");
-    if (!(out_flags & (TSB_OUT_WAVE | TSB_OUT_STATS))) return fail(ctx, TSB_E_INVALID, "no output selected");
+    if (!(out_flags & (TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_MEAS))) return fail(ctx, TSB_E_INVALID, "no output selected");
+    if ((rc = check_measures(b, TSB_AN_AC, out_flags)) != TSB_OK) return rc;
+    if (out_flags & TSB_OUT_MEAS) out_flags |= TSB_OUT_STATS;
     std::vector<double> f;
     ac_frequency_points(sweep_type, n_points, fstart, fstop, f);       // ac.go:100-126
     tsb_opts o = resolve(opts, p);
     o.coop_parts = 0;          // the cooperative mapping is a transient-only specialisation
-    fit_block_to_shared_memory(o, b->plan->p.num_columns(TSB_AN_AC), out_flags);
+    fit_block_to_shared_memory(o, b->plan->p.num_columns(TSB_AN_AC), out_flags, (int)b->meas.size());
     CU(ctx, cudaSetDevice(ctx->device));
     KernelModule* m = nullptr;
-    if ((rc = get_module(b, o, -1, &m)) != TSB_OK) return rc;
+    b->meas_kernel = (out_flags & TSB_OUT_MEAS) != 0;
+    rc = get_module(b, o, -1, &m);
+    b->meas_kernel = false;
+    if (rc != TSB_OK) return rc;
     if ((rc = alloc_results(b, TSB_AN_AC, out_flags, (out_flags & TSB_OUT_WAVE) ? (int64_t)n_points : 0, n_points)) != TSB_OK) return rc;
     TsbArgsHost a;
     if ((rc = fill_common(b, o, a)) != TSB_OK) return rc;
@@ -1381,6 +1436,31 @@ int tsb_batch_set_order(tsb_batch* b, const int64_t* perm) {
     static_assert(sizeof(long long) == sizeof(int64_t), "order entries are 64-bit");
     CU(ctx, cudaMemcpyAsync(b->d_order, perm, (size_t)b->n_inst * sizeof(long long), cudaMemcpyHostToDevice, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return TSB_OK;
+}
+
+int tsb_batch_set_measures(tsb_batch* b, const tsb_meas* m, int n_meas) {
+    if (!b || n_meas < 0 || (n_meas > 0 && !m)) return TSB_E_INVALID;
+    if (n_meas > TSB_MEAS_CAP) return fail(b->ctx, TSB_E_INVALID, "tsb_batch_set_measures: at most 16 measurements");
+    std::vector<tsb_meas> t(m, m + n_meas);
+    for (int k = 0; k < n_meas; ++k) {
+        tsb_meas& e = t[k];
+        const std::string at = "tsb_batch_set_measures: measurement " + std::to_string(k) + ": ";
+        if (e.kind < TSB_MEAS_WHEN || e.kind > TSB_MEAS_RMS) return fail(b->ctx, TSB_E_INVALID, at + "unknown kind");
+        if (e.column < 1) return fail(b->ctx, TSB_E_INVALID, at + "column must be >= 1 (column 0 is the abscissa)");
+        if (std::isnan(e.from) || std::isnan(e.to) || e.from > e.to) return fail(b->ctx, TSB_E_INVALID, at + "window needs from <= to");
+        if (e.kind == TSB_MEAS_WHEN) {
+            if (e.trig_column < 1) return fail(b->ctx, TSB_E_INVALID, at + "trig_column must be >= 1");
+            if (e.edge < TSB_EDGE_CROSS || e.edge > TSB_EDGE_FALL) return fail(b->ctx, TSB_E_INVALID, at + "unknown edge");
+            if (e.count == 0 || e.count < -1) return fail(b->ctx, TSB_E_INVALID, at + "count must be >= 1 or -1 (the last crossing)");
+        } else {
+            e.trig_column = e.column; e.edge = 0; e.count = 1;      // unused: kept out of the kernel specialisation
+        }
+        if ((e.kind == TSB_MEAS_WHEN || e.kind == TSB_MEAS_AT) && std::isnan(e.level)) return fail(b->ctx, TSB_E_INVALID, at + "level is NaN");
+    }
+    b->meas = t;
+    b->meas_last = 0;                  // the last run's results belong to the old table
+    b->memo_module = nullptr;
     return TSB_OK;
 }
 
@@ -1488,6 +1568,11 @@ int tsb_result_wave_all(tsb_batch* b, double* out, int64_t n_doubles) {
     return d2h(b, out, b->d_wave, b->wave_bytes);
 }
 int tsb_result_stats_all(tsb_batch* b, double* out) { return b && out ? d2h(b, out, b->d_stats, b->stats_bytes) : TSB_E_INVALID; }
+int tsb_result_measures(tsb_batch* b, double* out) {
+    if (!b || !out) return TSB_E_INVALID;
+    if (!b->meas_last) return fail(b->ctx, TSB_E_INVALID, "the last run had no TSB_OUT_MEAS");
+    return d2h(b, out, b->d_meas, (size_t)2 * b->meas_last * b->n_inst * sizeof(double));
+}
 int tsb_result_waveform(tsb_batch* b, int64_t inst, double* out, int64_t cap_rows, int64_t* n_rows) {
     int rc = check_batch(b); if (rc != TSB_OK) return rc;
     tsb_ctx* ctx = b->ctx;
@@ -1638,7 +1723,8 @@ int tsb_batch_kernel_variant(tsb_batch* b, int dc_src_dev, int dc_src2_dev, int 
     };
     int p1 = -1, p2 = -1;
     if (!param_of(dc_src_dev, &p1) || !param_of(dc_src2_dev, &p2)) return fail(b->ctx, TSB_E_INVALID, "source not found");
-    b->intro_dc_param = p1; b->dc_param2 = p2; b->dc_nested = dc_src2_dev >= 0; b->grid_kernel = grid != 0;
+    b->intro_dc_param = p1; b->dc_param2 = p2; b->dc_nested = dc_src2_dev >= 0;
+    b->grid_kernel = (grid & ~TSB_OUT_MEAS) != 0; b->meas_kernel = (grid & TSB_OUT_MEAS) != 0;
     b->memo_module = nullptr;
     return TSB_OK;
 }

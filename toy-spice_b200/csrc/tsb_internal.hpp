@@ -146,6 +146,7 @@ struct CodegenConfig {
     bool skip_linear = true;        // compile the redundant second linear solve away
     std::string extra_defines;      // development knob: extra #define lines ($TSB_EXTRA_DEFINES, ';'-separated NAME=VALUE)
     bool grid = false;              // kernels that carry the TSB_OUT_GRID resampling code
+    std::vector<int> meas;          // TSB_OUT_MEAS kernels: {kind, column, trigger column} per measurement; empty: none
     bool order = false;             // kernels that map launch slots to instances through a processing order
     bool lane_refill = false;       // nonlinear circuits: resident grid, finished lanes fetch the next instance
     bool tgrid = false;             // linear circuits: kernels that can read / publish the shared time grid (skeleton.cuh)
