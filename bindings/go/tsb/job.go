@@ -20,6 +20,7 @@ type Job struct {
 	h     *C.tsb_job
 	N     int64
 	nMeas int
+	nFour int
 }
 
 func NewJob(gpus []int, netlistText string, n int64) (*Job, error) {
@@ -110,6 +111,33 @@ func (j *Job) Measures() (value, abscissa [][]float64, err error) {
 		abscissa[m] = flat[int64(j.nMeas+m)*j.N : int64(j.nMeas+m+1)*j.N]
 	}
 	return value, abscissa, nil
+}
+
+// SetFourier sets the Fourier table of every GPU's shard.
+func (j *Job) SetFourier(f []Four) error {
+	t, rows := fourTable(f)
+	var p *C.tsb_four
+	if len(t) > 0 {
+		p = &t[0]
+	}
+	if rc := C.tsb_job_set_fourier(j.h, p, C.int(len(t))); rc != C.TSB_OK {
+		return j.err("tsb_job_set_fourier")
+	}
+	j.nFour = rows
+	return nil
+}
+
+// Fourier returns coeff[row][instance] in job order.
+func (j *Job) Fourier() ([][]float64, error) {
+	flat := make([]float64, int64(j.nFour)*j.N+1)
+	if rc := C.tsb_job_result_fourier(j.h, (*C.double)(unsafe.Pointer(&flat[0]))); rc != C.TSB_OK {
+		return nil, j.err("tsb_job_result_fourier")
+	}
+	out := make([][]float64, j.nFour)
+	for r := range out {
+		out[r] = flat[int64(r)*j.N : int64(r+1)*j.N]
+	}
+	return out, nil
 }
 
 func (j *Job) Status() ([]int32, error) {

@@ -145,6 +145,7 @@ type Batch struct {
 	plan  *Plan
 	N     int64
 	nMeas int
+	nFour int // output rows of the Fourier table, sum (1 + 2 NHarm)
 }
 
 func NewBatch(plan *Plan, n int64) (*Batch, error) {
@@ -271,6 +272,51 @@ func (b *Batch) Measures() (value, abscissa [][]float64, err error) {
 		abscissa[m] = flat[int64(b.nMeas+m)*b.N : int64(b.nMeas+m+1)*b.N]
 	}
 	return value, abscissa, nil
+}
+
+// Four is one entry of a Fourier table (tsb_four; the .four card, defined in tspice_b200.h).  TEnd = math.Inf(1): the
+// period that ends at tstop.
+type Four struct {
+	Column, NHarm, NGrid int
+	Freq, TEnd           float64
+}
+
+func fourTable(f []Four) ([]C.tsb_four, int) {
+	t := make([]C.tsb_four, len(f))
+	rows := 0
+	for k, e := range f {
+		t[k] = C.tsb_four{column: C.int(e.Column), n_harm: C.int(e.NHarm), n_grid: C.int(e.NGrid), freq: C.double(e.Freq),
+			t_end: C.double(e.TEnd)}
+		rows += 1 + 2*e.NHarm
+	}
+	return t, rows
+}
+
+// SetFourier sets the batch's Fourier table (copied; nil clears); runs with TSB_OUT_FOUR reduce it on the device.
+func (b *Batch) SetFourier(f []Four) error {
+	t, rows := fourTable(f)
+	var p *C.tsb_four
+	if len(t) > 0 {
+		p = &t[0]
+	}
+	if rc := C.tsb_batch_set_fourier(b.h, p, C.int(len(t))); rc != C.TSB_OK {
+		return b.plan.ctx.lastErr("tsb_batch_set_fourier")
+	}
+	b.nFour = rows
+	return nil
+}
+
+// Fourier returns coeff[row][instance] of the last TSB_OUT_FOUR run: per entry a0, A_1, B_1, ..., A_H, B_H.
+func (b *Batch) Fourier() ([][]float64, error) {
+	flat := make([]float64, int64(b.nFour)*b.N+1)
+	if rc := C.tsb_result_fourier(b.h, (*C.double)(unsafe.Pointer(&flat[0]))); rc != C.TSB_OK {
+		return nil, b.plan.ctx.lastErr("tsb_result_fourier")
+	}
+	out := make([][]float64, b.nFour)
+	for r := range out {
+		out[r] = flat[int64(r)*b.N : int64(r+1)*b.N]
+	}
+	return out, nil
 }
 
 // Stats returns min / max / sum / last per column and instance: stats[q][column][instance] (TSB_OUT_STATS runs).

@@ -159,7 +159,10 @@ enum {
                            source is not available, so both read-outs are offered (DESIGN.md, quirk Q28). */,
     TSB_OUT_MEAS = 16   /* tsb_run_tran / tsb_run_dc / tsb_run_ac: the measurements of the batch's measurement table
                            (tsb_batch_set_measures), reduced on the device from the stored rows as they are produced;
-                           read with tsb_result_measures.  Implies TSB_OUT_STATS; combines with WAVE and GRID. */
+                           read with tsb_result_measures.  Implies TSB_OUT_STATS; combines with WAVE and GRID. */,
+    TSB_OUT_FOUR = 32   /* tsb_run_tran only: the Fourier coefficients of the batch's Fourier table (tsb_batch_set_fourier),
+                           reduced on the device from the stored rows as they are produced; read with tsb_result_fourier.
+                           Implies TSB_OUT_STATS; combines with WAVE, GRID and MEAS. */
 };
 
 /* ---- measurements (the SPICE .meas family, reduced on the device) -------------------------------------------------
@@ -199,6 +202,37 @@ typedef struct tsb_meas {
     double level;      /* WHEN: crossing level; AT: the abscissa */
     double from, to;   /* window on column 0; -inf / +inf = the whole series */
 } tsb_meas;
+
+/* ---- Fourier analysis (the SPICE .four card, reduced on the device) -------------------------------------------------
+ * An entry {column, n_harm = H, n_grid = G, freq = f, t_end} reads the same series as a measurement: the instance's stored
+ * rows (x_r, y_r) of the transient, rows beyond wave_cap_rows included; y is `column`.
+ *   1. Window and grid, each step one IEEE double operation on the host: T = 1.0 / f; e = t_end, or the run's tstop when
+ *      t_end = +inf; s = e - T; D = T / G.  On the device tau_k = s + k D (k = 0 .. G-1) as two rounded operations:
+ *      __dadd_rn(s, __dmul_rn((double)k, D)).
+ *   2. y_k is the value of the series at tau_k as AT defines it: the first row with x >= tau_k; its y if x == tau_k,
+ *      else the interpolation between that row and the one before it.  If tau_0 < x_0 or tau_{G-1} > x_last (a window
+ *      before tstart, an instance that failed before the window ended or whose operating point failed) EVERY coefficient
+ *      of the entry is NaN.  A NaN sample propagates into the sums.
+ *   3. Twiddles c[j] = cos(2.0 * pi * j / G), s[j] = sin(2.0 * pi * j / G), j = 0 .. G-1, computed on the host with libm
+ *      (evaluated left to right, pi = M_PI) and indexed by (h k) mod G in integer arithmetic.
+ *   4. Sums from 0.0 over ascending k, every operation rounded on its own (no contraction, in both builds):
+ *      S0 = sum y_k, Ca_h = sum y_k c[(h k) mod G], Sb_h = sum y_k s[(h k) mod G].
+ *   5. Output 1 + 2H values per entry: a0 = S0 / G, A_h = (2.0 Ca_h) / G, B_h = (2.0 Sb_h) / G for h = 1 .. H, so that
+ *      y(tau) ~ a0 + sum_h A_h cos(2 pi h (tau - s) / T) + B_h sin(2 pi h (tau - s) / T).
+ *   6. Magnitude M_h = hypot(A_h, B_h), phase atan2(A_h, B_h) 180 / pi (of a sine referenced to the window start) and
+ *      THD = sqrt(sum_{h >= 2} M_h^2) / M_1 are left to the host (toy-spice_b200.fourier_summary).
+ * Column and H are compiled into the kernels (a new set compiles once, NVRTC); f, G and t_end are run-time arguments.
+ * Refused (before anything is launched): TSB_OUT_FOUR without a table or with a column outside 1 .. n_columns-1 of the
+ * transient (TSB_E_INVALID); on tsb_run_op / _dc / _dc2 / _ac or with an explicit coop_parts > 0 (TSB_E_UNSUPPORTED);
+ * coop_parts = -1 takes the thread-per-circuit mapping. */
+enum { TSB_FOUR_CAP = 8, TSB_FOUR_MAX_HARM = 32, TSB_FOUR_MAX_GRID = 65536 };
+typedef struct tsb_four {
+    int column;        /* result column analysed, 1 .. n_columns-1 of the transient (tsb_plan_column_name) */
+    int n_harm;        /* H, 1 .. 32 */
+    int n_grid;        /* G, 2H + 1 .. 65536 */
+    double freq;       /* fundamental frequency f, finite and > 0 */
+    double t_end;      /* end of the one-period window; +inf = the run's tstop */
+} tsb_four;
 
 void tsb_default_opts(tsb_opts* o);
 const char* tsb_version(void);
@@ -292,6 +326,12 @@ int tsb_batch_set_order(tsb_batch* batch, const int64_t* perm);
  * of the last run (tsb_result_measures fails until the next TSB_OUT_MEAS run). */
 int tsb_batch_set_measures(tsb_batch* batch, const tsb_meas* m, int n_meas);
 
+/* Fourier table of the batch (copied; n <= TSB_FOUR_CAP; (NULL, 0) clears).  TSB_E_INVALID, with no change of state, for
+ * a column < 1, n_harm outside 1 .. 32, n_grid outside 2 n_harm + 1 .. 65536, a freq that is not finite and > 0, and a
+ * t_end that is NaN or -inf.  The columns are checked against the transient when a run selects TSB_OUT_FOUR.  Setting a
+ * table discards the coefficients of the last run (tsb_result_fourier fails until the next TSB_OUT_FOUR run). */
+int tsb_batch_set_fourier(tsb_batch* batch, const tsb_four* f, int n);
+
 /* Analyses — the batch equivalents of analysis.NewOP / NewTransient / NewDCSweep + Setup + Execute. */
 int tsb_run_op(tsb_batch* batch, const tsb_opts* opts);
 int tsb_run_tran(tsb_batch* batch, double tstart, double tstop, double tstep, double tmax, int uic,
@@ -349,6 +389,9 @@ int tsb_result_stats_all(tsb_batch* batch, double* out /*[4][n_columns][n_inst]*
 /* Measurements of the last run (TSB_OUT_MEAS): out[0][m][inst] = value, out[1][m][inst] = abscissa, for the table the run
  * used.  TSB_E_INVALID after a run without measurements. */
 int tsb_result_measures(tsb_batch* batch, double* out /*[2][n_meas][n_inst]*/);
+/* Fourier coefficients of the last run (TSB_OUT_FOUR): out[k][inst], k running over the entries in table order with
+ * 1 + 2 n_harm rows each: a0, A_1, B_1, ..., A_H, B_H.  TSB_E_INVALID after a run without TSB_OUT_FOUR. */
+int tsb_result_fourier(tsb_batch* batch, double* out /*[sum (1 + 2 n_harm)][n_inst]*/);
 /* Batch totals computed on the GPU: sum over instances of accepted steps, rejected steps, transient solves,
  * OP solves (reference-equivalent counts) and executed factor+solve passes. */
 int tsb_result_totals(tsb_batch* batch, int64_t totals[5]);
@@ -387,6 +430,8 @@ int tsb_job_result_rows(tsb_job* job, int64_t* rows /*[n_inst]*/);
 int tsb_job_result_stats(tsb_job* job, double* stats /*[4][n_columns][n_inst]*/);
 int tsb_job_set_measures(tsb_job* job, const tsb_meas* m, int n_meas);
 int tsb_job_result_measures(tsb_job* job, double* out /*[2][n_meas][n_inst], JOB order*/);
+int tsb_job_set_fourier(tsb_job* job, const tsb_four* f, int n);
+int tsb_job_result_fourier(tsb_job* job, double* out /*[sum (1 + 2 n_harm)][n_inst], JOB order*/);
 int tsb_job_result_waveform(tsb_job* job, int64_t inst, double* out, int64_t cap_rows, int64_t* n_rows);
 /* out[3][n_columns] (min, max, sum), stored rows and the five totals of tsb_result_totals, merged over the GPUs. */
 int tsb_job_result_summary(tsb_job* job, double* out, int64_t* rows_total, int64_t totals[5]);
@@ -447,7 +492,8 @@ int tsb_batch_kernel_source(tsb_batch* batch, const tsb_opts* opts, char* buf, i
 /* Which specialisation the two calls below describe: dc_src_dev >= 0 selects the DC-sweep kernel for that source
  * (dc_src2_dev >= 0: the nested sweep), grid != 0 the TSB_OUT_GRID kernels; (-1, -1, 0) = the default OP / transient
  * kernels.  The bit TSB_OUT_MEAS in `grid` selects the kernels of the batch's measurement table instead (grid ==
- * TSB_OUT_MEAS) or in addition (grid == TSB_OUT_GRID | TSB_OUT_MEAS).  A batch used this way is for introspection only (build step), do not run analyses on it. */
+ * TSB_OUT_MEAS) or in addition (grid == TSB_OUT_GRID | TSB_OUT_MEAS); the bit TSB_OUT_FOUR likewise selects the kernels of
+ * its Fourier table, and grid & ~(TSB_OUT_MEAS | TSB_OUT_FOUR) decides the grid kernels.  A batch used this way is for introspection only (build step), do not run analyses on it. */
 int tsb_batch_kernel_variant(tsb_batch* batch, int dc_src_dev, int dc_src2_dev, int grid);
 /* Cache key (hex) of that source + compile options; the cubin is looked up as <cache_dir>/<key>.cubin. */
 int tsb_batch_kernel_key(tsb_batch* batch, const tsb_opts* opts, char* buf, int cap);

@@ -94,6 +94,18 @@ public:
         if (tsb_result_measures(h_, out.data()) != TSB_OK) throw Error(ckt_->ctx().last_error());
         return out;
     }
+    // Fourier table (TSB_OUT_FOUR; definitions in tspice_b200.h); an empty vector clears it.
+    void SetFourier(const std::vector<tsb_four>& f) {
+        if (tsb_batch_set_fourier(h_, f.empty() ? nullptr : f.data(), (int)f.size()) != TSB_OK) throw Error(ckt_->ctx().last_error());
+        four_rows_ = 0;
+        for (const tsb_four& e : f) four_rows_ += 1 + 2 * e.n_harm;
+    }
+    // [sum (1 + 2 n_harm)][n_inst] of the last run with TSB_OUT_FOUR: per entry a0, A_1, B_1, ..., A_H, B_H.
+    std::vector<double> Fourier() const {
+        std::vector<double> out((size_t)four_rows_ * n_);
+        if (tsb_result_fourier(h_, out.data()) != TSB_OK) throw Error(ckt_->ctx().last_error());
+        return out;
+    }
     tsb_batch* get() const { return h_; }
     Circuit& circuit() const { return *ckt_; }
     int64_t size() const { return n_; }
@@ -101,6 +113,7 @@ private:
     Circuit* ckt_;
     int64_t n_;
     int n_meas_ = 0;
+    int four_rows_ = 0;
     tsb_batch* h_ = nullptr;
 };
 
@@ -164,7 +177,7 @@ class Transient : public Analysis {
 public:
     Transient(double tStart, double tStop, double tStep, double tMax, bool uic)
         : tStart_(tStart), tStop_(tStop), tStep_(tStep), tMax_(tMax), uic_(uic) {}
-    int out = TSB_OUT_WAVE;      // TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_GRID (results resampled onto a fixed time grid) | TSB_OUT_MEAS
+    int out = TSB_OUT_WAVE;      // TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_GRID (results resampled onto a fixed time grid) | TSB_OUT_MEAS | TSB_OUT_FOUR
     int64_t cap_rows = 16384;
     double grid_dt = 0.0;        // TSB_OUT_GRID: grid spacing (0: the clamped tStep)
     void Execute() override {

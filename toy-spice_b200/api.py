@@ -26,7 +26,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
 
 AN_OP, AN_TRAN, AN_AC, AN_DC, AN_DC2 = 0, 1, 2, 3, 4
-OUT_WAVE, OUT_STATS, OUT_GRID, OUT_AC_REFREAD, OUT_MEAS = 1, 2, 4, 8, 16
+OUT_WAVE, OUT_STATS, OUT_GRID, OUT_AC_REFREAD, OUT_MEAS, OUT_FOUR = 1, 2, 4, 8, 16, 32
 MEAS_WHEN, MEAS_AT, MEAS_MAX, MEAS_MIN, MEAS_AVG, MEAS_INTEG, MEAS_RMS = range(7)
 EDGE_CROSS, EDGE_RISE, EDGE_FALL = range(3)
 K_R, K_C, K_L, K_V, K_I, K_D, K_Q, K_M, K_K, K_LCORE = range(10)
@@ -51,7 +51,8 @@ ABI_SYMBOLS = [
     "tsb_job_run_dc", "tsb_job_sync", "tsb_job_result_status", "tsb_job_result_rows", "tsb_job_result_stats",
     "tsb_job_result_waveform", "tsb_job_result_summary", "tsb_run_ac", "tsb_plan_analysis2",
     "tsb_lu_solve_batched_complex", "tsb_lu_solve_batched_complex_dev", "tsb_batch_set_measures", "tsb_result_measures",
-    "tsb_job_set_measures", "tsb_job_result_measures",
+    "tsb_job_set_measures", "tsb_job_result_measures", "tsb_batch_set_fourier", "tsb_result_fourier", "tsb_job_set_fourier",
+    "tsb_job_result_fourier",
 ]
 
 
@@ -80,6 +81,44 @@ def meas(kind: int, column: int, level: float = 0.0, trig_column: int | None = N
 def _meas_table(measures):
     arr = (Meas * max(1, len(measures)))(*measures)
     return (arr if measures else None), len(measures)
+
+
+class Four(C.Structure):
+    """One entry of a Fourier table (tsb_four; definitions in include/tspice_b200.h)."""
+    _fields_ = [("column", C.c_int), ("n_harm", C.c_int), ("n_grid", C.c_int), ("freq", C.c_double), ("t_end", C.c_double)]
+
+
+def four(column: int, freq: float, n_harm: int = 9, n_grid: int = 200, t_end: float = np.inf) -> Four:
+    """A Fourier-table entry: harmonics 1 .. n_harm of `column` over the period 1/freq that ends at t_end (+inf: tstop),
+    sampled at n_grid points."""
+    return Four(column, n_harm, n_grid, freq, t_end)
+
+
+def _four_table(entries):
+    arr = (Four * max(1, len(entries)))(*entries)
+    return (arr if entries else None), len(entries)
+
+
+def fourier_summary(coeffs, table):
+    """Per entry of `table` (list of Four), from the coefficients [sum (1 + 2H)][n_inst] of Batch.fourier(): a dict with
+    a0 [n_inst], M [H][n_inst] = hypot(A_h, B_h), phase_deg [H][n_inst] = atan2(A_h, B_h) 180 / pi (a sine's phase,
+    referenced to the window start) and thd [n_inst] = sqrt(sum_{h >= 2} M_h^2) / M_1."""
+    coeffs = np.asarray(coeffs, dtype=np.float64)
+    out, r = [], 0
+    for f in table:
+        H = f.n_harm
+        blk = coeffs[r:r + 1 + 2 * H]
+        A, B = blk[1::2], blk[2::2]
+        M = np.hypot(A, B)
+        with np.errstate(divide="ignore", invalid="ignore"):
+            thd = np.sqrt(np.sum(M[1:] ** 2, axis=0)) / M[0]
+        out.append(dict(a0=blk[0], M=M, phase_deg=np.degrees(np.arctan2(A, B)), thd=thd))
+        r += 1 + 2 * H
+    return out
+
+
+def _four_rows(table):
+    return sum(1 + 2 * f.n_harm for f in table)
 
 
 def lib_path() -> str:
@@ -150,6 +189,10 @@ def lib():
             "tsb_result_measures": (i32, [vp, P(dbl)]),
             "tsb_job_set_measures": (i32, [vp, P(Meas), i32]),
             "tsb_job_result_measures": (i32, [vp, P(dbl)]),
+            "tsb_batch_set_fourier": (i32, [vp, P(Four), i32]),
+            "tsb_result_fourier": (i32, [vp, P(dbl)]),
+            "tsb_job_set_fourier": (i32, [vp, P(Four), i32]),
+            "tsb_job_result_fourier": (i32, [vp, P(dbl)]),
             "tsb_result_totals": (i32, [vp, P(i64)]),
             "tsb_batch_kernel_source": (i32, [vp, P(Opts), C.c_char_p, i64, P(i64)]),
             "tsb_batch_kernel_key": (i32, [vp, P(Opts), C.c_char_p, i32]),
@@ -520,12 +563,12 @@ class Batch:
             self._check(lib().tsb_batch_set_param(self.h, d, param, v.ctypes.data_as(C.POINTER(C.c_double))), "set_param")
 
     # -- kernel introspection -------------------------------------------------------------------
-    def kernel_variant(self, dc_src=-1, dc_src2=-1, grid=False, meas=False):
+    def kernel_variant(self, dc_src=-1, dc_src2=-1, grid=False, meas=False, four=False):
         """Select the specialisation kernel_source / kernel_key describe (introspection-only batches; build step);
-        meas=True: the kernels of the batch's measurement table."""
+        meas=True / four=True: the kernels of the batch's measurement / Fourier table."""
         d1 = self._dev(dc_src) if dc_src != -1 else -1
         d2 = self._dev(dc_src2) if dc_src2 != -1 else -1
-        flags = (1 if grid else 0) | (OUT_MEAS if meas else 0)
+        flags = (1 if grid else 0) | (OUT_MEAS if meas else 0) | (OUT_FOUR if four else 0)
         self._check(lib().tsb_batch_kernel_variant(self.h, d1, d2, flags), "tsb_batch_kernel_variant")
 
     def kernel_source(self, opts: Opts | None = None) -> str:
@@ -641,6 +684,19 @@ class Batch:
         self._check(lib().tsb_result_measures(self.h, out.ctypes.data_as(C.POINTER(C.c_double))), "result_measures")
         return out
 
+    def set_fourier(self, table):
+        """Fourier table (tsb_batch_set_fourier): a list of Four (see four()); [] clears.  Runs with OUT_FOUR use it."""
+        self.four_table = []
+        tab, n = _four_table(list(table))
+        self._check(lib().tsb_batch_set_fourier(self.h, tab, n), "tsb_batch_set_fourier")
+        self.four_table = list(table)
+
+    def fourier(self) -> np.ndarray:
+        """[sum (1 + 2H)][n_inst] of the last run (OUT_FOUR): per entry a0, A_1, B_1, ..., A_H, B_H."""
+        out = np.zeros((_four_rows(getattr(self, "four_table", [])), self.n_inst))
+        self._check(lib().tsb_result_fourier(self.h, out.ctypes.data_as(C.POINTER(C.c_double))), "result_fourier")
+        return out
+
     def fetch_async(self, stats=None, rows=None, status=None, counters=None):
         """tsb_result_fetch_async: queue device -> host copies of the last run's results into (pinned) numpy arrays; they
         overlap later launches on the context and are complete after sync()."""
@@ -719,6 +775,19 @@ class Job:
         """[2: value, abscissa][n_meas][n_inst] in job order."""
         out = np.zeros((2, getattr(self, "n_meas", 0), self.n_inst))
         self._check(lib().tsb_job_result_measures(self.h, out.ctypes.data_as(C.POINTER(C.c_double))), "job_result_measures")
+        return out
+
+    def set_fourier(self, table):
+        """Fourier table of every shard (tsb_job_set_fourier)."""
+        self.four_table = []
+        tab, n = _four_table(list(table))
+        self._check(lib().tsb_job_set_fourier(self.h, tab, n), "job_set_fourier")
+        self.four_table = list(table)
+
+    def fourier(self) -> np.ndarray:
+        """[sum (1 + 2H)][n_inst] in job order."""
+        out = np.zeros((_four_rows(getattr(self, "four_table", [])), self.n_inst))
+        self._check(lib().tsb_job_result_fourier(self.h, out.ctypes.data_as(C.POINTER(C.c_double))), "job_result_fourier")
         return out
 
     def run_op(self, opts: Opts | None = None):

@@ -31,6 +31,24 @@ static const char* k_coop_src =
 #include "coop_src.inc"
     ;
 
+// The skeleton without its `#if TSB_FOUR` ... `#endif` blocks (nesting counted): kernels without a Fourier table are
+// generated from exactly the text they had before the table existed, so their source, cache key and code stay put.
+static std::string strip_four_blocks(const char* src) {
+    std::istringstream in(src);
+    std::string out, line;
+    int depth = 0;                       // > 0: inside a Fourier block, at this #if nesting depth
+    while (std::getline(in, line)) {
+        if (depth == 0 && line.rfind("#if TSB_FOUR", 0) == 0) { depth = 1; continue; }
+        if (depth > 0) {
+            if (line.rfind("#if", 0) == 0) ++depth;
+            else if (line.rfind("#endif", 0) == 0) --depth;
+            continue;
+        }
+        out += line; out += '\n';
+    }
+    return out;
+}
+
 namespace {
 
 std::string dlit(double v) {
@@ -975,8 +993,16 @@ std::string generate_source(const Plan& pl, const CodegenConfig& cfg) {
         e.line("#define TSB_MEAS " + std::to_string(cfg.meas.size() / 3));
         e.line("#define TSB_MEAS_SPEC " + spec);
     }
+    if (!cfg.four.empty()) {             // Fourier table: the compile-time half (skeleton.cuh, TsbSink::emit_four)
+        std::string spec;
+        for (size_t k = 0; k + 1 < cfg.four.size(); k += 2)
+            spec += (k ? ", {" : "{") + std::to_string(cfg.four[k]) + ", " + std::to_string(cfg.four[k + 1]) + "}";
+        e.line("#define TSB_FOUR " + std::to_string(cfg.four.size() / 2));
+        e.line("#define TSB_FOUR_SPEC " + spec);
+    }
     if (!cfg.extra_defines.empty()) e.os << cfg.extra_defines << "\n";     // development knob ($TSB_EXTRA_DEFINES)
-    e.os << k_models_src << "\n" << k_skeleton_src << "\n";
+    static const std::string skeleton_plain = strip_four_blocks(k_skeleton_src);
+    e.os << k_models_src << "\n" << (cfg.four.empty() ? skeleton_plain.c_str() : k_skeleton_src) << "\n";
 
     e.line("struct Ckt {");
     ++e.ind;

@@ -75,6 +75,16 @@ struct TsbArgs {
     double meas_level[16], meas_from[16], meas_to[16];
     int meas_count[16], meas_edge[16];
     double* meas_out;          // [2][n_meas][n_inst]: value, abscissa
+#if TSB_FOUR
+    // TSB_OUT_FOUR (kernels generated with TSB_FOUR): the run-time half of the Fourier table — column and number of
+    // harmonics are compile-time (tsb_four_spec).  Appended after meas_out: every field above keeps its offset.  The host
+    // always passes them; kernels without a table declare the struct without them and read its prefix.
+    double four_s[8], four_dt[8];   // window start s and grid spacing T / G of entry e
+    int four_g[8];                  // G
+    int four_tw_off[8];             // entry e's twiddles: four_tw[off .. off + G) cosines, [off + G .. off + 2G) sines
+    const double* four_tw;
+    double* four_out;               // [sum (1 + 2H)][n_inst]: the sums while the run accumulates, the coefficients after it
+#endif
 };
 
 // Slot -> instance.  With an order, lanes of a warp can be given instances that behave alike (similar Newton
@@ -191,6 +201,26 @@ __device__ __forceinline__ double tsb_meas_interp(double x0, double y0, double x
     return __dadd_rn(y0, __dmul_rn(__ddiv_rn(__dsub_rn(L, x0), __dsub_rn(x1, x0)), __dsub_rn(y1, y0)));
 }
 #endif
+#if TSB_FOUR
+// Fourier analysis (TSB_OUT_FOUR, the SPICE .four card; definitions in include/tspice_b200.h).  Kernels generated for a
+// Fourier table define TSB_FOUR (its length) and TSB_FOUR_SPEC ({column, harmonics} per entry).  Every line of it sits in
+// an `#if TSB_FOUR` block, which the code generator leaves out of kernels without a table: their source stays the same.
+#define TSB_OUT_FOUR 32
+struct TsbFourSpec { int col, harm; };
+__host__ __device__ constexpr TsbFourSpec tsb_four_spec(int i) {
+    constexpr TsbFourSpec t[TSB_FOUR] = {TSB_FOUR_SPEC};
+    return t[i];
+}
+// first output row of entry e: the entries before it take 1 + 2H rows each
+__host__ __device__ constexpr int tsb_four_row(int e) { return e == 0 ? 0 : tsb_four_row(e - 1) + 1 + 2 * tsb_four_spec(e - 1).harm; }
+#if !TSB_MEAS
+// a sample y_k is the series' value at tau_k as AT defines it: the interpolation of the measurement code above
+__device__ __forceinline__ double tsb_meas_interp(double x0, double y0, double x1, double y1, double L) {
+    if (L == x1) return y1;
+    return __dadd_rn(y0, __dmul_rn(__ddiv_rn(__dsub_rn(L, x0), __dsub_rn(x1, x0)), __dsub_rn(y1, y0)));
+}
+#endif
+#endif
 
 // Result sink of one instance: waveform rows to HBM (instance-fastest layout, so a warp whose
 // lanes are at the same row index writes 256 contiguous bytes per column) and running
@@ -223,7 +253,85 @@ struct TsbSink {
 #if TSB_MEAS
         if (a.out_flags & TSB_OUT_MEAS) meas_begin();
 #endif
+#if TSB_FOUR
+        if (a.out_flags & TSB_OUT_FOUR) four_begin();
+#endif
     }
+#if TSB_FOUR
+    // Entry e keeps one double2 per thread after the statistics and measurement pairs: {tau_k, k} of the next grid point
+    // k it waits for (tau = +inf once all G are taken).  A stored row costs one shared-memory load and one compare per
+    // entry; the sums live in place in four_out (instance-fastest rows, so a warp that takes a grid point together
+    // touches contiguous lines) and are read, updated and written at each of the G grid points.  Shared memory or
+    // registers for the 2H + 1 sums would cost residency or spills in the step loop (measured: DESIGN.md §5.2a).
+    __device__ __forceinline__ double2* four_slot(int e) const { return sm + (2 * NCOL + 2 * TSB_MEAS + e) * TSB_BLOCK; }
+    template <int e = 0> __device__ __forceinline__ void four_begin() {
+        if constexpr (e < TSB_FOUR) {
+            if constexpr (tsb_four_spec(e).col < NCOL) four_slot(e)[0] = make_double2(__dadd_rn(a.four_s[e], __dmul_rn(0.0, a.four_dt[e])), 0.0);
+            four_begin<e + 1>();
+        }
+    }
+    // One stored row, before the statistics update (the previous row is in the `last` slots): every grid point in
+    // (previous row, this row] is sampled and added into the sums.
+    template <int e = 0> __device__ __forceinline__ void emit_four(const double* row) {
+        if constexpr (e < TSB_FOUR) {
+            constexpr TsbFourSpec sp = tsb_four_spec(e);
+            if constexpr (sp.col < NCOL) {
+                double2* slot = four_slot(e);
+                const double x1 = row[0];
+                if (x1 >= slot[0].x) four_take<e>(x1, row[sp.col], slot);
+            }
+            emit_four<e + 1>(row);
+        }
+    }
+    template <int e> __device__ __forceinline__ void four_take(double x1, double y1, double2* slot) {
+        constexpr TsbFourSpec sp = tsb_four_spec(e);
+        const int G = a.four_g[e];
+        const double s = a.four_s[e], dt = a.four_dt[e];
+        const double* c = a.four_tw + a.four_tw_off[e];
+        const double* sn = c + G;
+        const double x0 = sm[1 * TSB_BLOCK].y, y0 = sm[(2 * sp.col + 1) * TSB_BLOCK].y;
+        double* o = a.four_out + (long long)tsb_four_row(e) * a.n_inst + inst;
+        int k = (int)slot[0].y;
+        double tk = slot[0].x;
+        while (x1 >= tk) {
+            // no row before this one: tau_0 < x_0 is outside the series, a NaN sample turns every sum NaN
+            const double y = n_rows > 0 ? tsb_meas_interp(x0, y0, x1, y1, tk) : (x1 == tk ? y1 : __longlong_as_double(0x7ff8000000000000LL));
+            const bool first = k == 0;                 // the sums start at 0.0: nothing to read yet
+            o[0] = __dadd_rn(first ? 0.0 : o[0], y);
+            int j = 0;
+#pragma unroll
+            for (int h = 1; h <= sp.harm; ++h) {
+                j += k; if (j >= G) j -= G;              // (h k) mod G
+                double* oh = o + (long long)(2 * h - 1) * a.n_inst;
+                oh[0] = __dadd_rn(first ? 0.0 : oh[0], __dmul_rn(y, __ldg(c + j)));
+                oh[a.n_inst] = __dadd_rn(first ? 0.0 : oh[a.n_inst], __dmul_rn(y, __ldg(sn + j)));
+            }
+            ++k;
+            tk = k < G ? __dadd_rn(s, __dmul_rn((double)k, dt)) : TSB_INF;
+        }
+        slot[0] = make_double2(tk, (double)k);
+    }
+    // coefficients from the sums; NaN for every row when a grid point was not reached (tau_{G-1} > x_last, no rows)
+    template <int e = 0> __device__ __forceinline__ void four_finish() {
+        if constexpr (e < TSB_FOUR) {
+            constexpr TsbFourSpec sp = tsb_four_spec(e);
+            if constexpr (sp.col < NCOL) {
+                const int G = a.four_g[e];
+                const bool all = (int)four_slot(e)[0].y == G;
+                const double g = (double)G;
+                double* o = a.four_out + (long long)tsb_four_row(e) * a.n_inst + inst;
+                const double nan = __longlong_as_double(0x7ff8000000000000LL);
+                o[0] = all ? __ddiv_rn(o[0], g) : nan;
+#pragma unroll
+                for (int r = 1; r <= 2 * sp.harm; ++r) {
+                    double* orow = o + (long long)r * a.n_inst;
+                    orow[0] = all ? __ddiv_rn(__dmul_rn(2.0, orow[0]), g) : nan;
+                }
+            }
+            four_finish<e + 1>();
+        }
+    }
+#endif
 #if TSB_MEAS
     // Measurement m keeps two double2 per thread after the statistics pairs (same thread-interleaved layout):
     //   WHEN            {value, abscissa} of the crossing taken, {crossings counted, -}
@@ -364,6 +472,9 @@ struct TsbSink {
 #if TSB_MEAS
         if (a.out_flags & TSB_OUT_MEAS) emit_meas(row);      // TSB_OUT_MEAS implies TSB_OUT_STATS: reads the `last` slots first
 #endif
+#if TSB_FOUR
+        if (a.out_flags & TSB_OUT_FOUR) emit_four(row);      // TSB_OUT_FOUR implies TSB_OUT_STATS: reads the `last` slots first
+#endif
         if (a.out_flags & TSB_OUT_STATS) {
             if (n_rows == 0) sm[0] = make_double2(row[0], row[0]);     // column 0: the first row, kept in the {min, max} slot
             // running min / max that ignore NaN samples (the accumulators start at +-inf and can never become NaN
@@ -417,6 +528,9 @@ struct TsbSink {
         }
 #if TSB_MEAS
         if (a.out_flags & TSB_OUT_MEAS) meas_finish();
+#endif
+#if TSB_FOUR
+        if (a.out_flags & TSB_OUT_FOUR) four_finish();
 #endif
         if (a.out_flags & TSB_OUT_STATS) {
 #pragma unroll

@@ -23,6 +23,7 @@ struct tsb_job {
     std::vector<Shard> shards;
     int64_t n_inst = 0;
     int n_meas = 0;                   // measurement table of every shard (tsb_job_set_measures)
+    int four_rows = 0;                // output rows of the Fourier table of every shard (tsb_job_set_fourier)
     std::string err;
 };
 
@@ -160,6 +161,31 @@ int tsb_job_result_measures(tsb_job* j, double* out) {
         const size_t rows = 2 * (size_t)j->n_meas;
         std::vector<double> tmp(rows * n);
         rc = tsb_result_measures(s.batch, tmp.data());
+        if (rc != TSB_OK) return rc;
+        for (size_t k = 0; k < rows; ++k) std::memcpy(out + k * j->n_inst + s.lo, tmp.data() + k * n, (size_t)n * sizeof(double));
+        return (int)TSB_OK;
+    });
+}
+int tsb_job_set_fourier(tsb_job* j, const tsb_four* f, int n) {
+    if (!j) return TSB_E_INVALID;
+    for (auto& s : j->shards) {
+        int rc = tsb_batch_set_fourier(s.batch, f, n);
+        if (rc != TSB_OK) return job_fail(j, rc, tsb_last_error(s.ctx));
+    }
+    j->four_rows = 0;
+    for (int k = 0; k < n; ++k) j->four_rows += 1 + 2 * f[k].n_harm;
+    return TSB_OK;
+}
+// Fourier coefficients [sum (1 + 2H)][n_inst] in job order (each shard's block is copied row by row into place)
+int tsb_job_result_fourier(tsb_job* j, double* out) {
+    if (!j || !out) return TSB_E_INVALID;
+    return for_all_shards(j, [&](tsb_job::Shard& s) {
+        int64_t n = 0;
+        int rc = tsb_result_dims(s.batch, &n, nullptr, nullptr);
+        if (rc != TSB_OK) return rc;
+        const size_t rows = (size_t)j->four_rows;
+        std::vector<double> tmp(rows * n);
+        rc = tsb_result_fourier(s.batch, tmp.data());
         if (rc != TSB_OK) return rc;
         for (size_t k = 0; k < rows; ++k) std::memcpy(out + k * j->n_inst + s.lo, tmp.data() + k * n, (size_t)n * sizeof(double));
         return (int)TSB_OK;

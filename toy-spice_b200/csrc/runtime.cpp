@@ -72,7 +72,12 @@ struct TsbArgsHost {
     double meas_level[16], meas_from[16], meas_to[16];
     int meas_count[16], meas_edge[16];
     double* meas_out;
+    double four_s[8], four_dt[8];
+    int four_g[8], four_tw_off[8];
+    const double* four_tw;
+    double* four_out;
 };
+static_assert(sizeof(TsbArgsHost) <= 4096, "the kernel argument block must stay within the 4 KB kernel-parameter limit");
 
 struct KernelModule {
     cudaLibrary_t lib = nullptr;
@@ -161,6 +166,15 @@ struct tsb_batch {
     double* d_meas = nullptr;                          // [2][n_meas][n_inst] of the last TSB_OUT_MEAS run
     size_t meas_bytes = 0;
     int meas_last = 0;                                 // measurements the last run produced (0: it had no TSB_OUT_MEAS)
+    std::vector<tsb_four> four;                        // tsb_batch_set_fourier
+    std::vector<double> four_tw;                       // its twiddles, per entry cos[G] then sin[G] (host libm)
+    bool four_tw_sent = false;                         // d_four_tw holds four_tw
+    bool four_kernel = false;                          // the next module request wants the kernels of this table (TSB_FOUR)
+    double* d_four = nullptr;                          // [sum (1 + 2H)][n_inst] of the last TSB_OUT_FOUR run
+    double* d_four_tw = nullptr;
+    size_t four_bytes = 0;
+    int four_last = 0;                                 // Fourier entries the last run produced (0: it had no TSB_OUT_FOUR)
+    int four_rows = 0;                                 // their output rows, sum (1 + 2H)
 };
 
 namespace {
@@ -291,6 +305,8 @@ CodegenConfig make_config(const tsb_batch* b, const tsb_opts& o, int dc_param) {
     cfg.grid = b->grid_kernel;
     if (b->meas_kernel)
         for (const tsb_meas& m : b->meas) { cfg.meas.push_back(m.kind); cfg.meas.push_back(m.column); cfg.meas.push_back(m.trig_column); }
+    if (b->four_kernel)
+        for (const tsb_four& f : b->four) { cfg.four.push_back(f.column); cfg.four.push_back(f.n_harm); }
     cfg.dc_nested = b->dc_nested; cfg.dc_param2 = b->dc_param2;
     cfg.order = b->d_order != nullptr;
     if (const char* x = getenv("TSB_EXTRA_DEFINES")) {          // development knob for A/B kernel experiments
@@ -370,6 +386,10 @@ int get_module(tsb_batch* b, tsb_opts o, int dc_param, KernelModule** out, std::
     sig += tail;
     if (b->meas_kernel)
         for (const tsb_meas& m : b->meas) sig += std::to_string(m.kind) + "," + std::to_string(m.column) + "," + std::to_string(m.trig_column) + ";";
+    if (b->four_kernel) {
+        sig += "|four:";
+        for (const tsb_four& f : b->four) sig += std::to_string(f.column) + "," + std::to_string(f.n_harm) + ";";
+    }
     if (xd) sig += xd;
     if (const char* tf = getenv("TSB_TRANFAST")) { sig += "|tf"; sig += tf; }
     if (b->memo_module && sig == b->memo_sig) {
@@ -476,7 +496,8 @@ int guard_check(tsb_batch* b) {
     auto name_of = [&](void* p) -> const char* {
         const std::pair<const void*, const char*> known[] = {
             {b->d_wave, "wave"}, {b->d_stats, "stats"}, {b->d_rows, "rows"}, {b->d_status, "status"},
-            {b->d_counters, "counters"}, {b->d_scratch, "scratch"}, {b->d_sweep, "sweep"}, {b->d_meas, "meas"}};
+            {b->d_counters, "counters"}, {b->d_scratch, "scratch"}, {b->d_sweep, "sweep"}, {b->d_meas, "meas"}, {b->d_four, "four"},
+            {b->d_four_tw, "four twiddles"}};
         for (const auto& kn : known)
             if (p == kn.first) return kn.second;
         return "buffer";
@@ -496,12 +517,13 @@ int guard_check(tsb_batch* b) {
 
 void free_results(tsb_batch* b) {
     gfree(b, b->d_wave); gfree(b, b->d_stats); gfree(b, b->d_rows); gfree(b, b->d_status);
-    gfree(b, b->d_counters); gfree(b, b->d_scratch); gfree(b, b->d_sweep); gfree(b, b->d_sweep2); gfree(b, b->d_meas); cudaFree(b->d_totals); cudaFree(b->d_work);
+    gfree(b, b->d_counters); gfree(b, b->d_scratch); gfree(b, b->d_sweep); gfree(b, b->d_sweep2); gfree(b, b->d_meas); gfree(b, b->d_four); gfree(b, b->d_four_tw); cudaFree(b->d_totals); cudaFree(b->d_work);
     b->d_work = nullptr;
     b->d_wave = b->d_stats = b->d_scratch = b->d_sweep = b->d_sweep2 = nullptr;
     b->d_rows = b->d_counters = nullptr; b->d_status = nullptr; b->d_totals = nullptr;
-    b->wave_bytes = b->stats_bytes = b->meas_bytes = 0;
-    b->meas_last = 0;
+    b->wave_bytes = b->stats_bytes = b->meas_bytes = b->four_bytes = 0;
+    b->meas_last = b->four_last = b->four_rows = 0;
+    b->four_tw_sent = false;
 }
 
 int alloc_results(tsb_batch* b, int analysis, int out_flags, int64_t cap_rows, int n_sweep) {
@@ -527,6 +549,25 @@ int alloc_results(tsb_batch* b, int analysis, int out_flags, int64_t cap_rows, i
             CU(ctx, galloc(b, (void**)&b->d_meas, meas_bytes)); b->meas_bytes = meas_bytes;
         }
         b->meas_last = (int)b->meas.size();
+    }
+    b->four_last = b->four_rows = 0;
+    if (out_flags & TSB_OUT_FOUR) {
+        int rows = 0;
+        for (const tsb_four& f : b->four) rows += 1 + 2 * f.n_harm;
+        const size_t four_bytes = (size_t)rows * N * sizeof(double);
+        if (four_bytes != b->four_bytes) {
+            gfree(b, b->d_four); b->four_bytes = 0;
+            CU(ctx, galloc(b, (void**)&b->d_four, four_bytes)); b->four_bytes = four_bytes;
+        }
+        if (!b->four_tw_sent) {          // once per table
+            gfree(b, b->d_four_tw);
+            CU(ctx, galloc(b, (void**)&b->d_four_tw, b->four_tw.size() * sizeof(double)));
+            CU(ctx, cudaMemcpyAsync(b->d_four_tw, b->four_tw.data(), b->four_tw.size() * sizeof(double), cudaMemcpyHostToDevice, ctx->stream));
+            CU(ctx, cudaStreamSynchronize(ctx->stream));     // a new table may replace the host copy
+            b->four_tw_sent = true;
+        }
+        b->four_last = (int)b->four.size();
+        b->four_rows = rows;
     }
     if (!b->d_rows) CU(ctx, galloc(b, (void**)&b->d_rows, N * sizeof(long long)));
     if (!b->d_status) CU(ctx, galloc(b, (void**)&b->d_status, N * sizeof(int)));
@@ -557,6 +598,7 @@ int launch(tsb_batch* b, const tsb_opts& o, cudaKernel_t kernel, TsbArgsHost& ar
     const int ncol_smem = b->plan->p.num_columns(b->analysis == TSB_AN_DC2 ? TSB_AN_DC2 : b->analysis == TSB_AN_AC ? TSB_AN_AC : TSB_AN_TRAN);
     size_t smem = (args.out_flags & (TSB_OUT_STATS | TSB_OUT_GRID)) ? (size_t)4 * ncol_smem * block * sizeof(double) : 0;
     if (args.out_flags & TSB_OUT_MEAS) smem += (size_t)4 * b->meas_last * block * sizeof(double);     // 32 bytes per measurement
+    if (args.out_flags & TSB_OUT_FOUR) smem += (size_t)2 * b->four_last * block * sizeof(double);     // 16 bytes per Fourier entry
     if (smem > 48 * 1024) CU(ctx, cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     long long blocks = (args.n_run + block - 1) / block;
     if (blocks > 0x7fffffffLL) blocks = 0x7fffffffLL;
@@ -642,10 +684,40 @@ tsb_opts resolve(const tsb_opts* o, const Plan& plan) {
 // Per-thread statistics live in shared memory (32 bytes per result column): a circuit with many result columns does not fit
 // 128 threads' worth into an SM's 227 KB.  The block shrinks (whole warps) until it does; the block size is part of the
 // kernel's specialisation, so this happens before the module is requested.
-void fit_block_to_shared_memory(tsb_opts& o, int ncol, int out_flags, int n_meas) {
+void fit_block_to_shared_memory(tsb_opts& o, int ncol, int out_flags, int n_meas, int n_four = 0) {
     if (!(out_flags & (TSB_OUT_STATS | TSB_OUT_GRID))) return;
-    const int slots = ncol + ((out_flags & TSB_OUT_MEAS) ? n_meas : 0);      // a measurement takes 32 bytes, as a column does
-    while (o.block_size > 32 && (size_t)4 * slots * o.block_size * sizeof(double) > (size_t)226 * 1024) o.block_size -= 32;
+    // a column and a measurement take 4 doubles per thread, a Fourier entry 2
+    const int per_thread = 4 * ncol + ((out_flags & TSB_OUT_MEAS) ? 4 * n_meas : 0) + ((out_flags & TSB_OUT_FOUR) ? 2 * n_four : 0);
+    while (o.block_size > 32 && (size_t)per_thread * o.block_size * sizeof(double) > (size_t)226 * 1024) o.block_size -= 32;
+}
+
+// TSB_OUT_FOUR: the table is checked against the transient's columns before anything is allocated or launched.
+int check_fourier(tsb_batch* b, int out_flags) {
+    if (!(out_flags & TSB_OUT_FOUR)) return TSB_OK;
+    if (b->four.empty()) return fail(b->ctx, TSB_E_INVALID, "TSB_OUT_FOUR: the batch has no Fourier table (tsb_batch_set_fourier)");
+    const int ncol = b->plan->p.num_columns(TSB_AN_TRAN);
+    for (const tsb_four& f : b->four)
+        if (f.column >= ncol)
+            return fail(b->ctx, TSB_E_INVALID, "TSB_OUT_FOUR: column " + std::to_string(f.column) + " is out of range for the transient (" +
+                                                   std::to_string(ncol) + " columns)");
+    return TSB_OK;
+}
+
+// TSB_OUT_FOUR: the run-time half of the table.  Window and grid as the header defines them, one IEEE operation per step.
+void fill_fourier(const tsb_batch* b, TsbArgsHost& a, double tstop) {
+    int off = 0;
+    for (int e = 0; e < b->four_last; ++e) {
+        const tsb_four& f = b->four[e];
+        const double T = 1.0 / f.freq;
+        const double end = std::isinf(f.t_end) ? tstop : f.t_end;
+        a.four_s[e] = end - T;
+        a.four_dt[e] = T / f.n_grid;
+        a.four_g[e] = f.n_grid;
+        a.four_tw_off[e] = off;
+        off += 2 * f.n_grid;
+    }
+    a.four_tw = b->d_four_tw;
+    a.four_out = b->d_four;
 }
 
 // TSB_OUT_MEAS: the table is checked against the columns of the analysis before anything is allocated or launched.
@@ -1159,11 +1231,12 @@ int tsb_run_tran(tsb_batch* b, double tstart, double tstop, double tstep, double
     int rc = check_batch(b); if (rc != TSB_OK) return rc;
     tsb_ctx* ctx = b->ctx;
     if (!(tstop > 0) || !(tstep > 0)) return fail(ctx, TSB_E_INVALID, "tstop and tstep must be positive");
-    if (!(out_flags & (TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_GRID | TSB_OUT_MEAS))) return fail(ctx, TSB_E_INVALID, "no output selected");
+    if (!(out_flags & (TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_GRID | TSB_OUT_MEAS | TSB_OUT_FOUR))) return fail(ctx, TSB_E_INVALID, "no output selected");
     if ((out_flags & TSB_OUT_WAVE) && (out_flags & TSB_OUT_GRID)) return fail(ctx, TSB_E_INVALID, "TSB_OUT_WAVE and TSB_OUT_GRID share the waveform buffer: select one");
     if ((out_flags & TSB_OUT_WAVE) && wave_cap_rows <= 0) return fail(ctx, TSB_E_INVALID, "wave_cap_rows must be positive");
     if ((rc = check_measures(b, TSB_AN_TRAN, out_flags)) != TSB_OK) return rc;
-    if (out_flags & TSB_OUT_MEAS) out_flags |= TSB_OUT_STATS;     // the previous stored row lives in the statistics' `last` slots
+    if ((rc = check_fourier(b, out_flags)) != TSB_OK) return rc;
+    if (out_flags & (TSB_OUT_MEAS | TSB_OUT_FOUR)) out_flags |= TSB_OUT_STATS;     // the previous stored row lives in the statistics' `last` slots
     tsb_opts o = resolve(opts, b->plan->p);
     // NewTransient (tran.go:29-55)
     if (tstep > tstop / 300) tstep = tstop / 300;
@@ -1189,7 +1262,7 @@ int tsb_run_tran(tsb_batch* b, double tstart, double tstop, double tstep, double
         // needs holds; otherwise thread-per-circuit
         const Plan& cpl = b->plan->p;
         o.coop_parts = 0;
-        if (!cpl.has_bjt && !cpl.has_mutual && !o.strict_fp && !(out_flags & (TSB_OUT_GRID | TSB_OUT_MEAS)) && o.skip_linear_resolve && !o.lane_refill) {
+        if (!cpl.has_bjt && !cpl.has_mutual && !o.strict_fp && !(out_flags & (TSB_OUT_GRID | TSB_OUT_MEAS | TSB_OUT_FOUR)) && o.skip_linear_resolve && !o.lane_refill) {
             // two parts where they fit; more parts only when the statistics of fewer do not leave an SM two blocks
             if (cpl.n() >= TSB_COOP_AUTO_MIN_N)
                 for (int pick : {2, 4, 8}) {
@@ -1208,21 +1281,24 @@ int tsb_run_tran(tsb_batch* b, double tstart, double tstop, double tstep, double
         if (o.strict_fp) return fail(ctx, TSB_E_UNSUPPORTED, "coop_parts: the nested-dissection order is a re-association, not available in the strict build");
         if (out_flags & TSB_OUT_GRID) return fail(ctx, TSB_E_UNSUPPORTED, "coop_parts: TSB_OUT_GRID is not available on the cooperative mapping");
         if (out_flags & TSB_OUT_MEAS) return fail(ctx, TSB_E_UNSUPPORTED, "coop_parts: TSB_OUT_MEAS is not available on the cooperative mapping");
+        if (out_flags & TSB_OUT_FOUR) return fail(ctx, TSB_E_UNSUPPORTED, "coop_parts: TSB_OUT_FOUR is not available on the cooperative mapping");
         if (!o.skip_linear_resolve || o.lane_refill) return fail(ctx, TSB_E_UNSUPPORTED, "coop_parts needs skip_linear_resolve = 1 and lane_refill = 0");
         if (o.min_blocks <= 0) o.min_blocks = 2;          // tsb_optran only runs the operating point here: no launch-bounds search
-    } else fit_block_to_shared_memory(o, b->plan->p.num_columns(TSB_AN_TRAN), out_flags, (int)b->meas.size());
+    } else fit_block_to_shared_memory(o, b->plan->p.num_columns(TSB_AN_TRAN), out_flags, (int)b->meas.size(), (int)b->four.size());
     KernelModule* m = nullptr;
     b->grid_kernel = (out_flags & TSB_OUT_GRID) != 0;
     b->meas_kernel = (out_flags & TSB_OUT_MEAS) != 0;
+    b->four_kernel = (out_flags & TSB_OUT_FOUR) != 0;
     std::string autokey;
     rc = get_module(b, o, -1, &m, &autokey);
-    if (rc != TSB_OK) { b->grid_kernel = b->meas_kernel = false; return rc; }
+    if (rc != TSB_OK) { b->grid_kernel = b->meas_kernel = b->four_kernel = false; return rc; }
     if ((rc = alloc_results(b, TSB_AN_TRAN, out_flags, (out_flags & (TSB_OUT_WAVE | TSB_OUT_GRID)) ? wave_cap_rows : 0, 0)) != TSB_OK) return rc;
     TsbArgsHost a;
     if ((rc = fill_common(b, o, a)) != TSB_OK) return rc;
     a.analysis = TSB_AN_TRAN; a.uic = uic;
     a.tstart = tstart; a.tstop = tstop; a.tstep = tstep; a.maxstep = tmax; a.minstep = minstep;
     a.grid_dt = grid_dt; a.n_grid = (int)n_grid;
+    if (out_flags & TSB_OUT_FOUR) fill_fourier(b, a, tstop);
     const bool persistent = b->plan->p.has_nonlinear && o.lane_refill != 0;
     const char* tune_env = getenv("TSB_AUTOTUNE");
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
@@ -1231,9 +1307,9 @@ int tsb_run_tran(tsb_batch* b, double tstart, double tstop, double tstep, double
         !(tune_env && *tune_env == '0') && cap == cudaStreamCaptureStatusNone) {
         rc = autotune_min_blocks(b, o, autokey, m->min_blocks, a, persistent);
         if (rc == TSB_OK) rc = get_module(b, o, -1, &m);
-        if (rc != TSB_OK) { b->grid_kernel = b->meas_kernel = false; return rc; }
+        if (rc != TSB_OK) { b->grid_kernel = b->meas_kernel = b->four_kernel = false; return rc; }
     }
-    b->grid_kernel = b->meas_kernel = false;
+    b->grid_kernel = b->meas_kernel = b->four_kernel = false;
     b->tgrid_used = 0;
     const Plan& pl = b->plan->p;
     if (o.coop_parts > 0) {
@@ -1286,6 +1362,7 @@ static int run_dc_impl(tsb_batch* b, int src_dev, double start, double stop, dou
         return fail(ctx, TSB_E_INVALID, nested ? "source not found" : "source not found");       // dc.go:47-68, :226-228
     if (!(inc > 0) || (nested && !(inc2 > 0))) return fail(ctx, TSB_E_INVALID, "sweep increment must be positive");
     if (out_flags & TSB_OUT_GRID) return fail(ctx, TSB_E_INVALID, "TSB_OUT_GRID applies to transient analysis only");
+    if (out_flags & TSB_OUT_FOUR) return fail(ctx, TSB_E_UNSUPPORTED, "TSB_OUT_FOUR applies to transient analysis only");
     if (!(out_flags & (TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_MEAS))) return fail(ctx, TSB_E_INVALID, "no output selected");
     if (nested && (out_flags & TSB_OUT_MEAS)) return fail(ctx, TSB_E_UNSUPPORTED, "TSB_OUT_MEAS: the nested DC sweep's column 0 is not monotone");
     if ((rc = check_measures(b, TSB_AN_DC, out_flags)) != TSB_OK) return rc;
@@ -1349,6 +1426,7 @@ int tsb_run_ac(tsb_batch* b, int sweep_type, int n_points, double fstart, double
                                              ":126-150); that state is an artefact of the un-vendored sparse module and is not reproduced");
     if (sweep_type < 0 || sweep_type > 2 || n_points < 1 || n_points > (1 << 20)) return fail(ctx, TSB_E_INVALID, "invalid sweep type or number of points");
     if (out_flags & TSB_OUT_GRID) return fail(ctx, TSB_E_INVALID, "TSB_OUT_GRID applies to transient analysis only");
+    if (out_flags & TSB_OUT_FOUR) return fail(ctx, TSB_E_UNSUPPORTED, "TSB_OUT_FOUR applies to transient analysis only");
     if (!(out_flags & (TSB_OUT_WAVE | TSB_OUT_STATS | TSB_OUT_MEAS))) return fail(ctx, TSB_E_INVALID, "no output selected");
     if ((rc = check_measures(b, TSB_AN_AC, out_flags)) != TSB_OK) return rc;
     if (out_flags & TSB_OUT_MEAS) out_flags |= TSB_OUT_STATS;
@@ -1464,6 +1542,34 @@ int tsb_batch_set_measures(tsb_batch* b, const tsb_meas* m, int n_meas) {
     return TSB_OK;
 }
 
+int tsb_batch_set_fourier(tsb_batch* b, const tsb_four* f, int n) {
+    if (!b || n < 0 || (n > 0 && !f)) return TSB_E_INVALID;
+    if (n > TSB_FOUR_CAP) return fail(b->ctx, TSB_E_INVALID, "tsb_batch_set_fourier: at most 8 entries");
+    std::vector<tsb_four> t(f, f + n);
+    std::vector<double> tw;
+    for (int k = 0; k < n; ++k) {
+        const tsb_four& e = t[k];
+        const std::string at = "tsb_batch_set_fourier: entry " + std::to_string(k) + ": ";
+        if (e.column < 1) return fail(b->ctx, TSB_E_INVALID, at + "column must be >= 1 (column 0 is TIME)");
+        if (e.n_harm < 1 || e.n_harm > TSB_FOUR_MAX_HARM) return fail(b->ctx, TSB_E_INVALID, at + "n_harm must be in 1 .. 32");
+        if (e.n_grid < 2 * e.n_harm + 1 || e.n_grid > TSB_FOUR_MAX_GRID) return fail(b->ctx, TSB_E_INVALID, at + "n_grid must be in 2 n_harm + 1 .. 65536");
+        if (!std::isfinite(e.freq) || !(e.freq > 0)) return fail(b->ctx, TSB_E_INVALID, at + "freq must be finite and positive");
+        if (std::isnan(e.t_end) || e.t_end == -INFINITY) return fail(b->ctx, TSB_E_INVALID, at + "t_end must be finite or +inf");
+        const size_t c0 = tw.size();
+        tw.resize(c0 + 2 * (size_t)e.n_grid);
+        for (int j = 0; j < e.n_grid; ++j) {           // evaluated left to right: ((2.0 pi) j) / G
+            tw[c0 + j] = std::cos(2.0 * M_PI * j / e.n_grid);
+            tw[c0 + e.n_grid + j] = std::sin(2.0 * M_PI * j / e.n_grid);
+        }
+    }
+    b->four = t;
+    b->four_tw = tw;
+    b->four_tw_sent = false;
+    b->four_last = b->four_rows = 0;   // the last run's results belong to the old table
+    b->memo_module = nullptr;
+    return TSB_OK;
+}
+
 int tsb_batch_sync(tsb_batch* b) {
     int rc = check_batch(b); if (rc != TSB_OK) return rc;
     CU(b->ctx, cudaSetDevice(b->ctx->device));
@@ -1572,6 +1678,11 @@ int tsb_result_measures(tsb_batch* b, double* out) {
     if (!b || !out) return TSB_E_INVALID;
     if (!b->meas_last) return fail(b->ctx, TSB_E_INVALID, "the last run had no TSB_OUT_MEAS");
     return d2h(b, out, b->d_meas, (size_t)2 * b->meas_last * b->n_inst * sizeof(double));
+}
+int tsb_result_fourier(tsb_batch* b, double* out) {
+    if (!b || !out) return TSB_E_INVALID;
+    if (!b->four_last) return fail(b->ctx, TSB_E_INVALID, "the last run had no TSB_OUT_FOUR");
+    return d2h(b, out, b->d_four, (size_t)b->four_rows * b->n_inst * sizeof(double));
 }
 int tsb_result_waveform(tsb_batch* b, int64_t inst, double* out, int64_t cap_rows, int64_t* n_rows) {
     int rc = check_batch(b); if (rc != TSB_OK) return rc;
@@ -1724,7 +1835,8 @@ int tsb_batch_kernel_variant(tsb_batch* b, int dc_src_dev, int dc_src2_dev, int 
     int p1 = -1, p2 = -1;
     if (!param_of(dc_src_dev, &p1) || !param_of(dc_src2_dev, &p2)) return fail(b->ctx, TSB_E_INVALID, "source not found");
     b->intro_dc_param = p1; b->dc_param2 = p2; b->dc_nested = dc_src2_dev >= 0;
-    b->grid_kernel = (grid & ~TSB_OUT_MEAS) != 0; b->meas_kernel = (grid & TSB_OUT_MEAS) != 0;
+    b->grid_kernel = (grid & ~(TSB_OUT_MEAS | TSB_OUT_FOUR)) != 0; b->meas_kernel = (grid & TSB_OUT_MEAS) != 0;
+    b->four_kernel = (grid & TSB_OUT_FOUR) != 0;
     b->memo_module = nullptr;
     return TSB_OK;
 }

@@ -147,6 +147,7 @@ struct CodegenConfig {
     std::string extra_defines;      // development knob: extra #define lines ($TSB_EXTRA_DEFINES, ';'-separated NAME=VALUE)
     bool grid = false;              // kernels that carry the TSB_OUT_GRID resampling code
     std::vector<int> meas;          // TSB_OUT_MEAS kernels: {kind, column, trigger column} per measurement; empty: none
+    std::vector<int> four;          // TSB_OUT_FOUR kernels: {column, harmonics} per Fourier entry; empty: none
     bool order = false;             // kernels that map launch slots to instances through a processing order
     bool lane_refill = false;       // nonlinear circuits: resident grid, finished lanes fetch the next instance
     bool tgrid = false;             // linear circuits: kernels that can read / publish the shared time grid (skeleton.cuh)
