@@ -458,7 +458,9 @@ int tsb_lu_order(int n, const double* A_nominal, int* pivot_row, int* pivot_col)
  * dense system after mat.Clear(); ckt.Stamp(status); mat.LoadGmin(gmin) on a freshly set-up circuit, status =
  * {Mode = mode (TSB_AN_OP or TSB_AN_TRAN), Time = time, TimeStep = dt, Gmin = gmin}, written to device memory as
  * A[inst][n][n] (row-major) and b[inst][n], 0-based = MNA index - 1.  With tsb_lu_solve_batched_dev and the plan's
- * own pivot order (tsb_plan_structure) it forms the two-kernel version of one Newton iteration.  Asynchronous. */
+ * own pivot order (tsb_plan_structure) it forms the two-kernel version of one Newton iteration.  Asynchronous.
+ * TSB_E_INVALID, before any launch: mode other than TSB_AN_OP / TSB_AN_TRAN, a null output pointer, or mode = TSB_AN_TRAN
+ * with dt not > 0 (zero, negative or NaN: the companion models divide by it). */
 int tsb_batch_stamp_dev(tsb_batch* batch, int mode, double time, double dt, double gmin, uint64_t A_dev, uint64_t b_dev,
                         const tsb_opts* opts);
 int tsb_lu_solve_batched(tsb_ctx* ctx, int n, const int* pivot_row, const int* pivot_col, const double* A, const double* b,

@@ -73,6 +73,111 @@ class Matrix:
         self.solution = np.concatenate([[0.0], x])
 
 
+# ------------------------------------------------------------------------------------------- Go's math where it is not libm's
+_SIN = (1.58962301576546568060e-10, -2.50507477628578072866e-8, 2.75573136213857245213e-6, -1.98412698295895385996e-4,
+        8.33333333332211858878e-3, -1.66666666666666307295e-1)
+_COS = (-1.13585365213876817300e-11, 2.08757008419747316778e-9, -2.75573141792967388112e-7, 2.48015872888517045348e-5,
+        -1.38888888888730564116e-3, 4.16666666666665929218e-2)
+
+
+def go_sin(x):
+    """math.Sin (Go src/math/sin.go; pure Go on amd64): Cody-Waite reduction by pi/4 in three parts and the Cephes
+    polynomials.  It differs from libm's sine in the last bit.  |x| >= 2^29 (Payne-Hanek in Go) is not restated: libm."""
+    if x == 0 or x != x:
+        return x
+    if math.isinf(x):
+        return math.nan
+    sign = x < 0
+    x = abs(x)
+    if x >= 536870912.0:
+        return -math.sin(x) if sign else math.sin(x)
+    j = int(x * 1.2732395447351626861510701069801148)         # 4/Pi, a Go constant: rounded once
+    y = float(j)
+    if j & 1:
+        j += 1
+        y += 1.0
+    j &= 7
+    z = ((x - y * 7.85398125648498535156e-1) - y * 3.77489470793079817668e-8) - y * 2.69515142907905952645e-15
+    if j > 3:
+        sign = not sign
+        j -= 4
+    zz = z * z
+    if j == 1 or j == 2:
+        c = _COS
+        y = 1.0 - 0.5 * zz + zz * zz * ((((((c[0] * zz) + c[1]) * zz + c[2]) * zz + c[3]) * zz + c[4]) * zz + c[5])
+    else:
+        c = _SIN
+        y = z + z * zz * ((((((c[0] * zz) + c[1]) * zz + c[2]) * zz + c[3]) * zz + c[4]) * zz + c[5])
+    return -y if sign else y
+
+
+def _is_odd_int(y):
+    return abs(y) < 2.0 ** 53 and y == math.floor(y) and int(y) % 2 == 1
+
+
+def go_pow(x, y):
+    """math.Pow (Go src/math/pow.go): the special cases, Sqrt for y = +-0.5, otherwise Exp(yf * Log(x)) for the fractional
+    part of |y| (yf in (-0.5, 0.5]) times the integer power by repeated squaring of the Frexp mantissa, one Ldexp at the
+    end — a few ulp from the correctly rounded power that libm's pow returns."""
+    if y == 0 or x == 1:
+        return 1.0
+    if y == 1:
+        return x
+    if x != x or y != y:
+        return math.nan
+    if x == 0:
+        if y < 0:
+            return -math.inf if math.copysign(1.0, x) < 0 and _is_odd_int(y) else math.inf
+        return x if math.copysign(1.0, x) < 0 and _is_odd_int(y) else 0.0
+    if math.isinf(y):
+        if x == -1:
+            return 1.0
+        return 0.0 if (abs(x) < 1) == (y > 0) else math.inf
+    if math.isinf(x):
+        if x < 0:
+            return go_pow(1 / x, -y)
+        return 0.0 if y < 0 else math.inf
+    if y == 0.5:
+        return math.sqrt(x) if x >= 0 else math.nan
+    if y == -0.5:
+        return 1 / math.sqrt(x) if x > 0 else math.nan
+    yf, yi = math.modf(abs(y))
+    if yf != 0 and x < 0:
+        return math.nan
+    if yi >= 2.0 ** 63:
+        if x == -1:
+            return 1.0
+        return 0.0 if (abs(x) < 1) == (y > 0) else math.inf
+    a1, ae = 1.0, 0
+    if yf != 0:
+        if yf > 0.5:
+            yf -= 1
+            yi += 1
+        a1 = math.exp(yf * math.log(x))
+    x1, xe = math.frexp(x)
+    i = int(yi)
+    while i != 0:
+        if xe < -(1 << 12) or (1 << 12) < xe:
+            ae += xe
+            break
+        if i & 1:
+            a1 *= x1
+            ae += xe
+        x1 *= x1
+        xe <<= 1
+        if x1 < 0.5:
+            x1 += x1
+            xe -= 1
+        i >>= 1
+    if y < 0:
+        a1 = math.copysign(math.inf, a1) if a1 == 0 else 1 / a1
+        ae = -ae
+    try:
+        return math.ldexp(a1, ae)
+    except OverflowError:
+        return math.copysign(math.inf, a1)
+
+
 def _v(voltages, node):
     return voltages[node] if node != 0 else 0.0
 
@@ -205,7 +310,7 @@ class Source:
         if self.stype == 0:
             return p[0]
         if self.stype == 1:
-            return p[0] + p[1] * math.sin(2.0 * PI * p[2] * t + p[3] * PI / 180.0)
+            return p[0] + p[1] * go_sin(2.0 * PI * p[2] * t + p[3] * PI / 180.0)
         if self.stype == 2:                                         # :179-209
             v1, v2, delay, rise, fall, pw, per = p
             if t < delay:
@@ -287,7 +392,7 @@ class Diode:                                                        # diode.go
         vt = _vt(temp)
         ratio = temp / (KELVIN + 27)
         egfact = -self.Eg / (2 * vt) * (temp / (KELVIN + 27) - 1.0)
-        return self.Is * math.pow(ratio, self.Xti / self.N) * math.exp(egfact)
+        return self.Is * go_pow(ratio, self.Xti / self.N) * math.exp(egfact)
 
     def Stamp(self, m, st):                                         # :184-227
         nvt = self.N * _vt(st.Temp)
@@ -434,7 +539,7 @@ class Mosfet:                                                       # mosfet.go
             eeff = vgst / (self.TOX * 100)
             ueff = self.UO
             if self.UCRIT > 0 and eeff > 0:
-                ueff /= (1.0 + math.pow(eeff / self.UCRIT, self.UEXP))
+                ueff /= (1.0 + go_pow(eeff / self.UCRIT, self.UEXP))
             vdsat = vgst
             if self.VMAX > 0:
                 ecrit = self.VMAX / ueff * 100
@@ -541,8 +646,8 @@ class Mosfet:                                                       # mosfet.go
             else:
                 qgs, qgd = cgs * self.vgs, cgd * self.vgd
             qgb = cgb * (self.vgs - self.vbs)
-            cbs = self.CBS / math.pow(1.0 - self.vbs / self.PB, self.MJ) if self.vbs < 0 else self.CBS * (1.0 + self.MJ * self.vbs / self.PB)
-            cbd = self.CBD / math.pow(1.0 - self.vbd / self.PB, self.MJ) if self.vbd < 0 else self.CBD * (1.0 + self.MJ * self.vbd / self.PB)
+            cbs = self.CBS / go_pow(1.0 - self.vbs / self.PB, self.MJ) if self.vbs < 0 else self.CBS * (1.0 + self.MJ * self.vbs / self.PB)
+            cbd = self.CBD / go_pow(1.0 - self.vbd / self.PB, self.MJ) if self.vbd < 0 else self.CBD * (1.0 + self.MJ * self.vbd / self.PB)
             qbs, qbd = cbs * self.vbs, cbd * self.vbd
             icgs, icgd, icgb, icbs, icbd = (qgs - 0.0) / dt, (qgd - 0.0) / dt, (qgb - 0.0) / dt, (qbs - 0.0) / dt, (qbd - 0.0) / dt
             if ng != 0:

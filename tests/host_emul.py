@@ -181,8 +181,9 @@ def _flat_parameters(ckt):
     return nominal, index
 
 
-def build(text, overrides, tmpdir, strict=True, dc_src=-1, dc_src2=-1, opts_kw=None, grid=False):
-    """g++-compile the kernel source of this netlist / set of per-instance parameters [/ swept source(s)]; returns (exe, info)."""
+def build(text, overrides, tmpdir, strict=True, dc_src=-1, dc_src2=-1, opts_kw=None, grid=False, main=None):
+    """g++-compile the kernel source of this netlist / set of per-instance parameters [/ swept source(s)]; returns (exe, info).
+    `main`: a driver of the caller's own in place of MAIN."""
     ckt = T.Circuit.from_netlist(text)
     b = ckt.batch(2)
     if dc_src != -1:
@@ -193,7 +194,7 @@ def build(text, overrides, tmpdir, strict=True, dc_src=-1, dc_src2=-1, opts_kw=N
         b.set_param(dev, par, np.resize(np.asarray(vals, dtype=np.float64), 2))      # (which parameters vary is what specialises the source)
     opts = T.default_opts(**{**dict(strict_fp=1 if strict else 0, min_blocks=1, block_size=32, share_time_grid=0, coop_parts=0), **(opts_kw or {})})
     src = b.kernel_source(opts)
-    key = (src, strict, tmpdir)
+    key = (src, strict, tmpdir, main)
     info = dict(ckt=ckt, opts=opts,
                 slots=[(int(s), int(k)) for k, s in re.findall(r"P\[(\d+)\] = __ldcs\(a\.pv\[(\d+)\]", src)],
                 ncol_max=int(re.search(r"NCOL_MAX = (\d+)", src).group(1)), n=int(re.search(r"static constexpr int N = (\d+)", src).group(1)))
@@ -206,7 +207,7 @@ def build(text, overrides, tmpdir, strict=True, dc_src=-1, dc_src2=-1, opts_kw=N
         host_src = src.replace("extern __shared__ double tsb_smem[];", "")
         for ptx, c in _ASM_HOST:
             host_src = host_src.replace(ptx, c)
-        f.write(SHIM + host_src + MAIN)
+        f.write(SHIM + host_src + (MAIN if main is None else main))
     flags = ["-O1", "-std=c++17", "-ffp-contract=off", "-w"] + ([] if strict else ["-DTSB_FAST_DIV"])
     r = subprocess.run(["g++"] + flags + ["-o", exe, cpp], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr[-4000:]

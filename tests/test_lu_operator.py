@@ -200,8 +200,10 @@ def test_two_kernel_newton_iteration_equals_the_fused_kernel(ctx, name):
 
 @pytest.mark.gpu
 def test_stamp_kernel_transient_companion_models(ctx):
-    """rc.cir in transient mode at (t, dt): G + C/dt and the source value, written by the stamp kernel."""
+    """rc.cir in transient mode at (t, dt): G + C/dt and the source value, written by the stamp kernel — bit for bit the
+    reference's system (tests/stamp_ref.py, whose CPU test holds it to the hand-written companion matrix)."""
     import torch
+    import stamp_ref as R
     n_inst = 257
     ckt = T.Circuit.from_netlist(T.BUNDLED["rc"], ctx)
     ov = PU.draws("rc", ckt, n_inst)
@@ -214,9 +216,6 @@ def test_stamp_kernel_transient_companion_models(ctx):
     b.stamp_dev(T.AN_TRAN, t, dt, 0.0, dA.data_ptr(), db.data_ptr(), opts=T.default_opts(strict_fp=1))
     b.sync(); torch.cuda.synchronize()
     A, rhs = dA.cpu().numpy(), db.cpu().numpy()
-    g = 1.0 / ov[("r1", 0)]; geq = ov[("c1", 0)] / dt
-    ref = np.zeros((n_inst, 3, 3))
-    ref[:, 0, 0] = g; ref[:, 0, 1] = -g; ref[:, 1, 0] = -g; ref[:, 1, 1] = g + geq; ref[:, 2, 0] = 1.0; ref[:, 0, 2] = 1.0
-    assert np.array_equal(A, ref)
-    assert np.array_equal(rhs[:, :2], np.zeros((n_inst, 2)))                      # fresh capacitor: charge1 = 0
-    assert np.allclose(rhs[:, 2], 5.0 * np.sin(2 * np.pi * 1000.0 * t), rtol=4e-16, atol=0)
+    ref = R.stamp_batch(R.Deck(T.BUNDLED["rc"]), ov, range(n_inst), R.TRAN, t, dt, 0.0)
+    assert np.array_equal(A.view(np.int64), ref.A.view(np.int64))
+    assert np.array_equal(rhs.view(np.int64), ref.b.view(np.int64))

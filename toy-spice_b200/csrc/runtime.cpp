@@ -1460,6 +1460,10 @@ int tsb_batch_stamp_dev(tsb_batch* b, int mode, double time, double dt, double g
     int rc = check_batch(b); if (rc != TSB_OK) return rc;
     tsb_ctx* ctx = b->ctx;
     if (!A_dev || !b_dev || (mode != 0 && mode != 1)) return fail(ctx, TSB_E_INVALID, "tsb_batch_stamp_dev: mode must be 0 (OP) or 1 (transient), outputs non-null");
+    // A transient stamp divides by the step (C/dt, M/dt, ...); the fast build multiplies by 1/dt instead, which the kernel
+    // only forms for dt > 0, so a zero, negative or NaN step would stamp those conductances as 0 there and as +-Inf or a
+    // negative conductance in the strict build.  No analysis takes such a step: refuse it.
+    if (mode == TSB_AN_TRAN && !(dt > 0)) return fail(ctx, TSB_E_INVALID, "tsb_batch_stamp_dev: transient mode needs dt > 0");
     tsb_opts o = resolve(opts, b->plan->p);
     o.coop_parts = 0;          // the cooperative mapping is a transient-only specialisation
     CU(ctx, cudaSetDevice(ctx->device));
